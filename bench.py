@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run, one rank per GPU)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --steps K --dump-outputs bench_outputs    (also writes the last timed step's results as bench_outputs/*.npy)
 
 Workload (BASELINE.json configs[1]): 100 synthetic profiles, chr21 (46,709,983 bp -> 1.56e6 windows of 30 bp), one
 read group each (30x, 2x150 bp, insert ~ N(500, 50^2)), planted deletions; per GPU one such window range (weak
@@ -247,6 +248,37 @@ def measured_peak_gbs():
     return 6650.0, "fallback 6.65 TB/s (B200_PROFILING.md)"
 
 
+DUMP_BYTES = 64 << 20
+
+
+def output_arrays(res, budget=DUMP_BYTES):
+    """What a caller of Scanner.scan() receives, as float64 arrays (exact for every field): each field of the calls, the
+    per-sample rows and, with the device-side merge, the significant-window counts. Beyond `budget` bytes a fixed, seeded
+    sample of the calls is kept; `call_index` says which. Copies: a scan(copy=False) result is overwritten by the next scan."""
+    calls, per, sig = res["calls"], res["per_sample"], res["significant_windows"]
+    n = len(calls)
+    row_bytes = 8 * (len(calls.dtype.names) + per[0].size + (sig is not None) + 1) if n else 8
+    rows = np.arange(n)
+    if n * row_bytes > budget - 4096:                                   # (4 kB for the .npy headers and the counts)
+        k = max(0, (budget - 4096) // row_bytes)
+        rows = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+    out = {f"calls_{f}": calls[f][rows] for f in calls.dtype.names}
+    out["per_sample"] = per[rows]
+    if sig is not None:
+        out["significant_windows"] = sig[rows]
+    out["call_index"] = rows
+    out["n_calls"] = np.array([n])
+    out["n_windows"] = np.array([res["n_windows"]])
+    out["n_window_calls"] = np.array([res["n_window_calls"]])
+    return {k: np.asarray(v, dtype=np.float64) for k, v in out.items()}
+
+
+def write_outputs(d, arrays):
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, f"{name}.npy"), a)
+
+
 # ----------------------------------------------------------------------------------------------------------------
 # our arm
 # ----------------------------------------------------------------------------------------------------------------
@@ -355,6 +387,7 @@ def run_ours(args, rank, world, local_rank):
         launches += int(res["n_kernel_launches"])
     barrier()
     dt = time.perf_counter() - t0
+    dumped = output_arrays(res) if args.dump_outputs and rank == 0 else None
     n_lines = len(clocks.lines)
     t_w = time.time()
     while clocks.proc and len(clocks.lines) == n_lines and time.time() - t_w < 1.0:   # keep the load up until the sampler has seen it
@@ -537,6 +570,8 @@ def run_ours(args, rank, world, local_rank):
         gc.collect()
         torch.cuda.empty_cache()
         out["e2e_files"] = e2e_files(args)
+    if dumped is not None:
+        write_outputs(args.dump_outputs, dumped)
     emit_json(out)
 
 
@@ -752,7 +787,15 @@ def main():
     ap.add_argument("--mixed", action="store_true", help="1-3 read groups per sample with mixed insert-size histograms")
     ap.add_argument("--device-gen", action="store_true", help="--shard-samples: generate the read pairs on the GPU (libpdsynth_cuda.so) and hand them "
                                                                "over with pd_contig_push_device (cohorts too large for the host generator)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (calls, per-sample rows, "
+                                                          "significant windows) as DIR/<name>.npy in float64, at most 64 MB in all. "
+                                                          "Window-range scan only: not with --impl reference (its output is VCF "
+                                                          "text) or --shard-samples (each rank holds only its own samples' rows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.shard_samples):
+        ap.error("--dump-outputs covers the window-range scan (the default --impl ours without --shard-samples)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
