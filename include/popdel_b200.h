@@ -170,8 +170,10 @@ int pd_contig_scan(pd_ctx * ctx, uint64_t first_window, uint64_t n_windows, pd_r
  * length / LR, chain of similar calls, median start and length, PLs summed over the variant's windows and
  * re-normalised, median LAD / DAD, allele frequency from the genotypes, CSWin filter bit 16) and returns only the
  * merged variants. Segments with a single window call, or without a passing one (unless output_failed), return
- * nothing, like the reference. pd_set_unify(ctx, NULL) switches back to window calls. Not available for
- * sample-sharded contexts. */
+ * nothing, like the reference. pd_set_unify(ctx, NULL) switches back to window calls. May be called before or after
+ * attaching a context to a sample-sharded cohort; every rank must then use the same settings (a collective scan whose ranks
+ * differ fails with PD_ERR_ARG on every rank before any kernel runs). Each rank returns the same merged variants, with
+ * the allele frequency over all n_samples_global samples, and per_sample holds the merged rows of its own samples. */
 typedef struct {
     double  mean_stddev;                   /* mean insert-size standard deviation over all read groups */
     double  min_relative_window_cover;     /* -c, default 0.5 */
@@ -192,7 +194,9 @@ int pd_contig_reserve_windows(pd_ctx * ctx, uint64_t n_windows);
  * pd_contig_scan is then a COLLECTIVE: all ranks call it with the same window range after pushing their read pairs
  * (and pd_contig_reserve_windows). It all-gathers the screen's tile flags, the per-window Q3 values and the contig
  * tail, and exchanges the EM's per-iteration sufficient statistics inside the EM kernels through peer memory
- * (NVLink). Every rank returns the same calls; per_sample holds the rows of the rank's own samples. */
+ * (NVLink). Every rank returns the same calls; per_sample holds the rows of the rank's own samples. With pd_set_unify
+ * on every rank the window calls stay on the devices: each rank merges them over its own samples and the ranks
+ * all-gather one allele count per merged variant for the frequency. */
 typedef struct {
     uint32_t rank, world;                  /* world = 2..8 */
     uint32_t n_samples_global;

@@ -326,7 +326,8 @@ class Scanner:
 
     def set_unify(self, mean_stddev=None, min_relative_window_cover: float = 0.5, output_failed: bool = False):
         """pd_set_unify: scans return the merged variants of every segment (unifyCalls, utils_popdel.h:567-654, run on the
-        device); mean_stddev=None switches back to window calls."""
+        device); mean_stddev=None switches back to window calls. On a sample-sharded scanner (attach_nccl, ShardGroup)
+        every rank must use the same settings: each rank then returns the cohort's variants with its own samples' rows."""
         if mean_stddev is None:
             self._check(self.lib.pd_set_unify(self.ctx, None))
             return
@@ -347,11 +348,14 @@ class Scanner:
         if n:
             C.memmove(calls.ctypes.data, res.calls, n * CALL_DTYPE.itemsize)
             C.memmove(per.ctypes.data, res.per_sample, per.nbytes)
+        sig = None
+        if res.significant_windows:
+            sig = np.ctypeslib.as_array(res.significant_windows, shape=(max(n, 1),))[:n].copy()
         return dict(calls=calls, per_sample=per, n_windows=res.n_windows, n_flagged_windows=res.n_flagged_windows,
                     n_candidates=res.n_candidates, n_reads=res.n_reads, algorithmic_bytes=res.algorithmic_bytes,
                     h2d_bytes=res.h2d_bytes, d2h_bytes=res.d2h_bytes, n_kernel_launches=res.n_kernel_launches,
                     ms_h2d=res.ms_h2d, ms_screen=res.ms_screen, ms_genotype=res.ms_genotype, ms_total=res.ms_total,
-                    ms_stream=res.ms_stream, significant_windows=None, n_window_calls=res.n_window_calls, ms_unify=res.ms_unify,
+                    ms_stream=res.ms_stream, significant_windows=sig, n_window_calls=res.n_window_calls, ms_unify=res.ms_unify,
                     ms_em=res.ms_em, n_em_pairs_timed=res.n_em_pairs_timed, n_screened_windows=res.n_screened_windows,
                     n_known_pairs=res.n_known_pairs)
 
@@ -560,52 +564,91 @@ def cohort_headers(samples):
                   hist_start=rg.hist_start, hist_end=rg.hist_end, hist_counts=rg.hist_counts) for rg in s.read_groups] for s in samples]
 
 
-def scan_cohort_sample_sharded(samples, params: CallParameters, world: int, devices=None, first_window: int = 0, n_windows: int = 0,
-                               contig_len: int = 0):
-    """Sample-sharded scan of an in-memory cohort with `world` contexts of THIS process (pd_shard_attach_group /
-    pd_shard_group_scan; devices[r] = GPU of rank r, default all on GPU 0). Returns the merged result (calls of rank 0,
-    per-sample rows concatenated in cohort order) and the read groups of the whole cohort."""
-    lib = load_library()
+def sample_shard_scanner(samples, params: CallParameters, world: int, rank: int, device: int = 0, contig_len: int = 0):
+    """Rank `rank` of a sample-sharded in-memory cohort: a Scanner holding the rank's block of samples (split_samples), its
+    read pairs pushed and the cohort's window range reserved, not yet attached. Returns (scanner, read groups of the whole
+    cohort, samples per rank, minInitDelLengths of the whole cohort): what attach_nccl / pd_shard_attach_group take."""
     rgs = read_groups_from_headers(cohort_headers(samples), params)                 # parameters of the WHOLE cohort
     spr = split_samples(len(samples), world)
-    devices = list(devices) if devices is not None else [0] * world
     mi = np.array([r.min_init_del_len for r in rgs], dtype=np.uint32)
-    sprs = np.array(spr, dtype=np.uint32)
     anchor = cohort_anchor(samples)
     if not contig_len:
         contig_len = max(int(rg.pos[-1]) + 25000 for s in samples for rg in s.read_groups if rg.pos.size)
-    scanners, s0 = [], 0
-    try:
-        for r in range(world):
-            mine = [g for g in rgs if s0 <= g.sample < s0 + spr[r]]
-            local = [ReadGroup(**{**g.__dict__, "sample": g.sample - s0}) for g in mine]
-            sc = Scanner(params, local, spr[r], devices[r])
-            scanners.append(sc)
-            sc.begin_contig(anchor)
-            sc.reserve_windows((contig_len - anchor) // 30 + 2)
-            gi = 0
-            for s in samples[s0:s0 + spr[r]]:
-                for rg in s.read_groups:
-                    sc.push(gi, rg.pos, rg.dev)
-                    gi += 1
-            s0 += spr[r]
-        ctxs = (C.c_void_p * world)(*[sc.ctx for sc in scanners])
-        infos = (PdShardInfo * world)(*[PdShardInfo(r, world, len(samples), mi.size, mi.ctypes.data_as(C.POINTER(C.c_uint32)),
-                                                    sprs.ctypes.data_as(C.POINTER(C.c_uint32))) for r in range(world)])
-        rc = lib.pd_shard_attach_group(ctxs, world, infos)
+    s0 = sum(spr[:rank])
+    local = [ReadGroup(**{**g.__dict__, "sample": g.sample - s0}) for g in rgs if s0 <= g.sample < s0 + spr[rank]]
+    sc = Scanner(params, local, spr[rank], device)
+    sc.begin_contig(anchor)
+    sc.reserve_windows((contig_len - anchor) // 30 + 2)
+    gi = 0
+    for s in samples[s0:s0 + spr[rank]]:
+        for rg in s.read_groups:
+            sc.push(gi, rg.pos, rg.dev)
+            gi += 1
+    return sc, rgs, spr, mi
+
+
+class ShardGroup:
+    """A sample-sharded in-memory cohort over `world` contexts of THIS process (pd_shard_attach_group; devices[r] = GPU of
+    rank r, default all on GPU 0). scan() is the collective pd_shard_group_scan and may be repeated; scanners[r].set_unify
+    changes what the next scan returns (the same settings on every rank)."""
+
+    def __init__(self, samples, params: CallParameters, world: int, devices=None, contig_len: int = 0):
+        self.lib = load_library()
+        devices = list(devices) if devices is not None else [0] * world
+        self.world, self.scanners = world, []
+        try:
+            for r in range(world):
+                sc, self.rgs, self.spr, mi = sample_shard_scanner(samples, params, world, r, devices[r], contig_len)
+                self.scanners.append(sc)
+            self.ctxs = (C.c_void_p * world)(*[sc.ctx for sc in self.scanners])
+            sprs = np.array(self.spr, dtype=np.uint32)
+            infos = (PdShardInfo * world)(*[PdShardInfo(r, world, len(samples), mi.size, mi.ctypes.data_as(C.POINTER(C.c_uint32)),
+                                                        sprs.ctypes.data_as(C.POINTER(C.c_uint32))) for r in range(world)])
+            self._check(self.lib.pd_shard_attach_group(self.ctxs, world, infos), "pd_shard_attach_group")
+        except BaseException:
+            self.close()
+            raise
+
+    def _check(self, rc, what):
         if rc != 0:
-            raise ScanError(f"[{rc}] pd_shard_attach_group: " + "; ".join(lib.pd_last_error(sc.ctx).decode() for sc in scanners))
-        outs = (PdResult * world)()
-        rc = lib.pd_shard_group_scan(ctxs, world, int(first_window), int(n_windows), outs)
-        if rc != 0:
-            raise ScanError(f"[{rc}] pd_shard_group_scan: " + "; ".join(lib.pd_last_error(sc.ctx).decode() for sc in scanners))
-        parts = [sc._result_dict(outs[r]) for r, sc in enumerate(scanners)]
+            raise ScanError(f"[{rc}] {what}: " + "; ".join(self.lib.pd_last_error(sc.ctx).decode() for sc in self.scanners))
+
+    def set_unify(self, *args, **kw):
+        """Scanner.set_unify on every rank."""
+        for sc in self.scanners:
+            sc.set_unify(*args, **kw)
+
+    def scan(self, first_window: int = 0, n_windows: int = 0) -> dict:
+        """The result of rank 0 with the per-sample rows of all ranks concatenated in cohort order; `parts` = every rank's
+        own result. The ranks must agree on the calls (and significant windows)."""
+        outs = (PdResult * self.world)()
+        self._check(self.lib.pd_shard_group_scan(self.ctxs, self.world, int(first_window), int(n_windows), outs), "pd_shard_group_scan")
+        parts = [sc._result_dict(outs[r]) for r, sc in enumerate(self.scanners)]
         for p in parts[1:]:
             assert np.array_equal(p["calls"], parts[0]["calls"]), "ranks disagree on the calls"
+            assert (p["significant_windows"] is None) == (parts[0]["significant_windows"] is None)
+            if p["significant_windows"] is not None:
+                assert np.array_equal(p["significant_windows"], parts[0]["significant_windows"]), "ranks disagree on the significant windows"
         merged = dict(parts[0])
         merged["per_sample"] = np.concatenate([p["per_sample"] for p in parts], axis=1)
         merged["parts"] = parts
-        return merged, rgs
-    finally:
-        for sc in scanners:
+        return merged
+
+    def close(self):
+        for sc in self.scanners:
             sc.close()
+
+
+def scan_cohort_sample_sharded(samples, params: CallParameters, world: int, devices=None, first_window: int = 0, n_windows: int = 0,
+                               contig_len: int = 0, unify: dict = None):
+    """Sample-sharded scan of an in-memory cohort with `world` contexts of THIS process (ShardGroup). Returns the combined
+    result (calls of rank 0, per-sample rows concatenated in cohort order) and the read groups of the whole cohort: window
+    calls, or -- with unify=dict(mean_stddev=..., min_relative_window_cover=..., output_failed=...) -- the merged variants,
+    the same on every rank, with the allele frequency over the whole cohort."""
+    g = ShardGroup(samples, params, world, devices, contig_len)
+    try:
+        if unify:
+            g.set_unify(**unify)
+        return g.scan(first_window, n_windows), g.rgs
+    finally:
+        g.close()

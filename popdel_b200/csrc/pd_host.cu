@@ -630,7 +630,6 @@ extern "C" int pd_set_unify(pd_ctx * c, const pd_unify_params * p)
     if (!c) return PD_ERR_ARG;
     if (c->status) return c->status;
     if (!p) { c->unify_on = false; return 0; }
-    if (c->shard) return pd_fail(c, PD_ERR_ARG, "pd_set_unify: not available for sample-sharded contexts (merge the gathered rows on the host)");
     if (!(p->mean_stddev >= 0) || !(p->min_relative_window_cover >= 0)) return pd_fail(c, PD_ERR_ARG, "pd_set_unify: negative or NaN parameter");
     c->unify = *p; c->unify_on = true;
     return 0;

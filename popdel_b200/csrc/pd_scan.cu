@@ -138,7 +138,6 @@ int pd_run_scan(pd_ctx * c, uint64_t first_window, uint64_t n_windows, pd_result
     const uint32_t Nb = sh ? sh->n_local_max : N, Rb = sh ? sh->r_global : R, Ng = sh ? sh->n_global : N;
     const size_t row = 13ull * N;
     const bool uni = c->unify_on;                                     // window calls stay on the device, merged there
-    if (uni && sh) return pd_fail(c, PD_ERR_ARG, "device-side unify is not available for sample-sharded contexts");
     if (ensure_results(c, 1, row, 0)) return c->status;
     if (uni && pd_unify_ensure_raw(c, 1, row, 0)) return c->status;
     c->res_count[0] = 0;

@@ -2,8 +2,9 @@
 // rank holds N/world samples of the SAME window range and the scan exchanges
 //   * the tile flags of the screen (all-gather + OR),
 //   * the per-(window, sample) Q3 values (all-gather; every rank then derives the same candidate lengths),
-//   * the last-window summary of the pushed read pairs (all-gather of 32 bytes),
-//   * the per-iteration EM sufficient statistics, inside the EM kernels through peer memory (pd_em_common.cuh).
+//   * the last-window summary of the pushed read pairs and the unify settings (all-gather of 64 bytes),
+//   * the per-iteration EM sufficient statistics, inside the EM kernels through peer memory (pd_em_common.cuh),
+//   * with pd_set_unify: the number of merged variants and one allele count per variant (pd_unify.cu).
 // Two transports for the all-gathers and for mapping the peers' exchange slots:
 //   NCCL  one process per GPU; the caller hands over an ncclUniqueId (pd_shard_unique_id on rank 0, distributed by
 //         whatever the launcher offers, e.g. torch.distributed); slots are mapped with CUDA IPC over NVLink. libnccl
@@ -187,20 +188,29 @@ int pd_shard_or_flags(pd_ctx * c, uint32_t * flags, uint32_t n, cudaStream_t st)
     return 0;
 }
 
-// number of windows the reference scans for the COHORT's contig: combines the ranks' tail summaries
+// number of windows the reference scans for the COHORT's contig: combines the ranks' tail summaries. The same exchange
+// carries every rank's unify settings (the first collective of a sharded scan): the unify stage has collectives of its
+// own, so a rank that merged while another did not would wait for it forever. On a difference every rank fails here,
+// before any kernel of the scan runs.
 int pd_shard_window_total(pd_ctx * c, uint64_t * total)
 {
     PdShard * s = c->shard;
-    int64_t mine[4] = {c->tail.kf, c->tail.S, c->tail.E, c->tail.E_spill};
-    int64_t all[4 * PD_MAX_WORLD];
-    PD_CUDA(c, cudaMemcpyAsync(s->d_small, mine, 32, cudaMemcpyHostToDevice, c->stream));
-    if (pd_shard_allgather(c, s->d_small, (char *)s->d_small + 1024, 32, c->stream)) return c->status;
-    PD_CUDA(c, cudaMemcpyAsync(all, (char *)s->d_small + 1024, 32 * s->world, cudaMemcpyDeviceToHost, c->stream));
+    int64_t mine[8] = {c->tail.kf, c->tail.S, c->tail.E, c->tail.E_spill, c->unify_on, 0, 0, 0};
+    if (c->unify_on) {
+        memcpy(&mine[5], &c->unify.mean_stddev, 8); memcpy(&mine[6], &c->unify.min_relative_window_cover, 8);
+        mine[7] = c->unify.output_failed != 0;
+    }
+    int64_t all[8 * PD_MAX_WORLD];
+    PD_CUDA(c, cudaMemcpyAsync(s->d_small, mine, 64, cudaMemcpyHostToDevice, c->stream));
+    if (pd_shard_allgather(c, s->d_small, (char *)s->d_small + 1024, 64, c->stream)) return c->status;
+    PD_CUDA(c, cudaMemcpyAsync(all, (char *)s->d_small + 1024, 64 * s->world, cudaMemcpyDeviceToHost, c->stream));
     PD_CUDA(c, cudaStreamSynchronize(c->stream));
+    for (uint32_t r = 1; r < s->world; ++r)
+        if (memcmp(all + 4, all + 8 * r + 4, 32) != 0) return pd_fail(c, PD_ERR_ARG, "sample-sharded scan: unify settings differ between ranks (pd_set_unify)");
     PdTail t;
-    for (uint32_t r = 0; r < s->world; ++r) t.kf = std::max(t.kf, all[4 * r]);
+    for (uint32_t r = 0; r < s->world; ++r) t.kf = std::max(t.kf, all[8 * r]);
     for (uint32_t r = 0; r < s->world; ++r) {
-        const int64_t * a = all + 4 * r;
+        const int64_t * a = all + 8 * r;
         if (a[0] < 0) continue;
         if (a[0] == t.kf) { t.S = std::max(t.S, a[1]); t.E = std::max(t.E, a[2]); }
         else if (a[0] == t.kf - 1) t.E = std::max(t.E, a[3]);

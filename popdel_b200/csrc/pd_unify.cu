@@ -18,17 +18,22 @@
 //   k_unify_emit     grid (variants, sample groups), one WARP per (variant, sample) with the lanes over the variant's
 //                    in-range windows: PL sums -> setGenotypes, median LAD / DAD by bisection on the value over the
 //                    column staged in shared memory, allele count -> frequency; header + row go to mapped host memory.
+//   k_unify_freq     sample-sharded cohorts only: the plan depends on the call headers alone, which every rank holds
+//                    identically, so every rank merges the same variants over its own samples' rows; the frequency then
+//                    takes the allele counts of all ranks (all-gathered) over the cohort's n_global samples.
 #include <algorithm>
 #include <cstdlib>
 #include <cstring>
 
 #include "pd_device.cuh"
+#include "pd_shard.h"
 
 namespace {
 
 struct UnifyArgs {
     const pd_call * calls; const uint32_t * ps;        // window calls of the scan (device), window order
     uint32_t n_raw, row_words, N, nseg;
+    uint32_t n_global;                                 // samples of the cohort (sample-sharded: all ranks; else N)
     double sd, min_cover; int output_failed;
     int force_global;                                  // test knob (PD_UNIFY_GLOBAL): run the merge loop on global memory
     uint32_t * seg_first, * seg_last;                  // [nseg]
@@ -333,6 +338,16 @@ __global__ void __launch_bounds__(EMIT_WARPS_U * 32) k_unify_emit(UnifyArgs u)
     }
 }
 
+// parts = [world][total] allele counts of the ranks; the expression is that of k_unify_emit with the cohort's sample count
+__global__ void k_unify_freq(UnifyArgs u, const uint32_t * __restrict__ parts, uint32_t total, uint32_t world)
+{
+    const uint32_t slot = blockIdx.x * blockDim.x + threadIdx.x;
+    if (slot >= total || u.gwc[u.vlist[slot]] == 0) return;      // kept without a merge: the window call's cohort frequency
+    uint32_t a = 0;
+    for (uint32_t r = 0; r < world; ++r) a += parts[(size_t)r * total + slot];
+    u.out_calls[slot].frequency = (double)a / (u.n_global * 2.0);
+}
+
 template <typename T>
 int grow(pd_ctx * c, int slot, T *& p, size_t need)
 {
@@ -345,6 +360,20 @@ int grow(pd_ctx * c, int slot, T *& p, size_t need)
         c->cap_unify[slot] = want;
     }
     p = reinterpret_cast<T *>(c->d_unify[slot]);
+    return 0;
+}
+
+// sample-sharded: all-gathers the variant count of every rank; fails on every rank when they differ
+int shard_agree_total(pd_ctx * c, uint32_t total)
+{
+    PdShard * s = c->shard;
+    uint32_t all[PD_MAX_WORLD];
+    PD_CUDA(c, cudaMemcpyAsync(s->d_small, &total, 4, cudaMemcpyHostToDevice, c->stream));
+    if (pd_shard_allgather(c, s->d_small, (char *)s->d_small + 1024, 4, c->stream)) return c->status;
+    PD_CUDA(c, cudaMemcpyAsync(all, (char *)s->d_small + 1024, 4 * s->world, cudaMemcpyDeviceToHost, c->stream));
+    PD_CUDA(c, cudaStreamSynchronize(c->stream));
+    for (uint32_t r = 0; r < s->world; ++r)
+        if (all[r] != total) return pd_fail(c, PD_ERR_ARG, "sample-sharded scan: ranks disagree on the merged variants");
     return 0;
 }
 
@@ -388,33 +417,43 @@ int pd_run_unify(pd_ctx * c, uint32_t n_raw, size_t row, uint32_t nseg, int (*en
                  uint64_t * n_out, uint64_t * launches)
 {
     *n_out = 0;
-    if (n_raw == 0) return 0;
+    PdShard * sh = c->shard;
+    if (n_raw == 0 && !sh) return 0;
     cudaStream_t st = c->stream;
     UnifyArgs u;
     memset(&u, 0, sizeof(u));
     u.calls = c->d_u_calls; u.ps = c->d_u_ps; u.n_raw = n_raw; u.row_words = (uint32_t)row; u.N = c->N; u.nseg = nseg;
+    u.n_global = sh ? sh->n_global : c->N;
     u.force_global = getenv("PD_UNIFY_GLOBAL") != nullptr;
     u.sd = c->unify.mean_stddev; u.min_cover = c->unify.min_relative_window_cover; u.output_failed = c->unify.output_failed;
-    if (grow(c, 0, u.seg_first, (size_t)nseg)) return c->status;
-    if (grow(c, 1, u.seg_last, (size_t)nseg)) return c->status;
-    if (grow(c, 2, u.seg_keep, (size_t)nseg + 1)) return c->status;
-    if (grow(c, 3, u.order, (size_t)n_raw)) return c->status;
-    if (grow(c, 4, u.wc, (size_t)n_raw)) return c->status;
-    if (grow(c, 5, u.starts, (size_t)n_raw)) return c->status;
-    if (grow(c, 6, u.sizes, (size_t)n_raw)) return c->status;
-    if (grow(c, 7, u.inr, (size_t)n_raw)) return c->status;
-    if (grow(c, 8, u.gwc, (size_t)n_raw)) return c->status;
-    if (grow(c, 9, u.sig, (size_t)n_raw)) return c->status;
-    u.total = c->res_count + 1;
-    PD_CUDA(c, cudaMemsetAsync(u.seg_first, 0, (size_t)nseg * 4, st));
-    PD_CUDA(c, cudaMemsetAsync(u.seg_last, 0, (size_t)nseg * 4, st));
-    k_seg_bounds<<<(n_raw + 255) / 256, 256, 0, st>>>(u);
-    k_unify_plan<<<nseg, 256, 0, st>>>(u);
-    k_unify_offsets<<<1, 1024, 0, st>>>(u);
-    *launches += 3;
-    PD_CUDA(c, cudaGetLastError());
-    PD_CUDA(c, cudaStreamSynchronize(st));
-    const uint32_t total = c->res_count[1];
+    // (sample-sharded: this stage starts after the rank's last EM chunk has completed, and that chunk only completes once
+    // every peer's last EM launch is running and has posted its statistics; no peer kernel waits for this rank any more, so
+    // the allocations below may synchronise the device -- the rule of pd_shard_prelaunch does not apply here)
+    if (n_raw) {
+        if (grow(c, 0, u.seg_first, (size_t)nseg)) return c->status;
+        if (grow(c, 1, u.seg_last, (size_t)nseg)) return c->status;
+        if (grow(c, 2, u.seg_keep, (size_t)nseg + 1)) return c->status;
+        if (grow(c, 3, u.order, (size_t)n_raw)) return c->status;
+        if (grow(c, 4, u.wc, (size_t)n_raw)) return c->status;
+        if (grow(c, 5, u.starts, (size_t)n_raw)) return c->status;
+        if (grow(c, 6, u.sizes, (size_t)n_raw)) return c->status;
+        if (grow(c, 7, u.inr, (size_t)n_raw)) return c->status;
+        if (grow(c, 8, u.gwc, (size_t)n_raw)) return c->status;
+        if (grow(c, 9, u.sig, (size_t)n_raw)) return c->status;
+        u.total = c->res_count + 1;
+        PD_CUDA(c, cudaMemsetAsync(u.seg_first, 0, (size_t)nseg * 4, st));
+        PD_CUDA(c, cudaMemsetAsync(u.seg_last, 0, (size_t)nseg * 4, st));
+        k_seg_bounds<<<(n_raw + 255) / 256, 256, 0, st>>>(u);
+        k_unify_plan<<<nseg, 256, 0, st>>>(u);
+        k_unify_offsets<<<1, 1024, 0, st>>>(u);
+        *launches += 3;
+        PD_CUDA(c, cudaGetLastError());
+        PD_CUDA(c, cudaStreamSynchronize(st));
+    }
+    const uint32_t total = n_raw ? c->res_count[1] : 0;
+    // every rank must enter the same exchanges: the plan depends on the (identical) call headers only, so the counts agree;
+    // if they do not, every rank fails here instead of some of them waiting for the allele exchange below
+    if (sh && shard_agree_total(c, total)) return c->status;
     if (total) {
         if (ensure_results(c, total, row, 0)) return c->status;
         if (total > c->cap_res_sig || !c->res_sig) {
@@ -437,6 +476,17 @@ int pd_run_unify(pd_ctx * c, uint32_t n_raw, size_t row, uint32_t nseg, int (*en
         k_unify_emit<<<dim3(total, gy), EMIT_WARPS_U * 32, 0, st>>>(u);
         *launches += 2;
         PD_CUDA(c, cudaGetLastError());
+        if (sh) {                                                 // allele counts of every rank -> the cohort's frequency
+            const size_t need = (size_t)total * 4 * sh->world;
+            if (need > sh->cap_recv) {
+                cudaFree(sh->d_recv); sh->d_recv = nullptr; sh->cap_recv = 0;
+                PD_CUDA(c, cudaMalloc(&sh->d_recv, need + need / 4)); sh->cap_recv = need + need / 4;
+            }
+            if (pd_shard_allgather(c, u.alleles, sh->d_recv, (size_t)total * 4, st)) return c->status;
+            k_unify_freq<<<(total + 255) / 256, 256, 0, st>>>(u, (const uint32_t *)sh->d_recv, total, sh->world);
+            *launches += 1;
+            PD_CUDA(c, cudaGetLastError());
+        }
         PD_CUDA(c, cudaStreamSynchronize(st));
     }
     *n_out = total;
