@@ -625,6 +625,9 @@ __device__ __forceinline__ void dl_one(const RgOne & k, const int32_t * cache_d,
     }
 }
 
+// read pairs per lane whose loads the final pass issues together
+constexpr int FINAL_BATCH = 2;
+
 template <int LPS, int SLOTS, int BATCH>
 __device__ __forceinline__ void em_one_body(const PdDev & a, const EmArgs & e, EmShared & sh, uint32_t * s_first, uint32_t * s_last,
                                             uint32_t & s_nsupp, uint16_t * s_perm, int32_t * cache_dev, double * s_slot)
@@ -839,39 +842,74 @@ __device__ __forceinline__ void em_one_body(const PdDev & a, const EmArgs & e, E
     const double l10_min_prob = __ldg(&a.rgc[has ? s : 0].l10_min_prob);
     const int delLower = usable ? flen - lower_q : INT_MAX, delUpper = usable ? flen + upper_q : 0;
     const uint32_t * pp = e.pool_pos + poff;
+    // the read pairs of a lane in batches of FINAL_BATCH, over the warp's largest count so that the batches stay warp-uniform
+    const int nlw = __reduce_max_sync(PD_FULL, nl);
     unsigned long long supp = 0, ndata = 0;
     {
         // The ln sums of the final overload (:255-337) equal those of the likelihood pass the registers hold (same read pairs,
         // length and shift: see the state machine above), so only the log10 sums, LAD / DAD and the positions are taken
-        // here, from the second half of the table rows {log10, log10p, val, fr}.
-        uint32_t lad0 = 0, lad1 = 0, lad2 = 0, dad0 = 0, dad1 = 0, dad2 = 0, dad3 = 0, dad4 = 0;
+        // here, from the second half of the table rows {log10, log10p, val, fr}. A batch issues all its deviation, table
+        // and position loads before any value-dependent branch; the log10 sums still add the read pairs of a lane in order.
+        // (lad1 and dad4 are what the other classes leave of the lane's nl read pairs: two registers fewer in the loop)
+        uint32_t lad0 = 0, lad2 = 0, dad0 = 0, dad1 = 0, dad2 = 0, dad3 = 0, nsp = 0;
         uint32_t fl_min = 0xFFFFFFFFu, fl_max = 0, ndeg = 0;
         double t0 = 0, t1 = 0, t2 = 0;
-        for (int j = 0; j < nl; ++j) {
-            const int d = j < SLOTS ? cache_dev[j * T + tid] : __ldg(pd + sub + j * LPS);
-            if (d > upper_q) { if (d < delLower) ++dad2; else if (d <= delUpper) ++dad3; else ++dad4; }
-            else { if (d < delUpper) ++dad0; else ++dad1; }
-            const PdTab * tr = k.fl + (tab_in(k, d - shift) ? d - shift + k.hist_base + 1 : 0);
-            const PdTab * td = k.fl + (tab_in(k, d - flen) ? d - flen + k.hist_base + 1 : 0);
-            const D4 r2 = ld4(&tr->l10);                                                                  // log10 ref, log10p, ref, fr
-            D4 d2 = D4{l10_min_prob, 0, k.min_prob, 0};                                                  // floor: .b / .d unused
-            if (td != k.fl) d2 = ld4(&td->l10);
-            const double ref = r2.c, del = d2.c;
-            if (ref >= 2 * del) ++lad0; else if (del >= 2 * ref) ++lad2; else ++lad1;
-            t0 += r2.a; t2 += d2.a;
-            if (ref == del) { t1 += r2.a; ++ndeg; }                                      // residue applied below
-            else if (del == k.min_prob) t1 += r2.b;
-            else if (ref == k.min_prob) t1 += d2.b;
-            else t1 += log10(ref + del) - LOG10_2_D;
-            const uint32_t first = __ldg(pp + sub + j * LPS) + e.anchor;
-            const uint32_t last = first + (uint32_t)max(0, d + inner_off);
-            fl_min = min(fl_min, first); fl_max = max(fl_max, last);
-            if (d >= delLower && d <= delUpper) {                                        // supporting read pair
-                ++supp;
-                const uint32_t slot = atomicAdd(&s_nsupp, 1u);
-                if (slot < SUPP_CAP) { s_first[slot] = first; s_last[slot] = last; }
+        const uint32_t lane_lt = (1u << (tid & 31)) - 1u;
+        for (int b = 0; b < nlw; b += FINAL_BATCH) {
+            int d[FINAL_BATCH]; uint32_t first[FINAL_BATCH]; D4 r2[FINAL_BATCH], d2[FINAL_BATCH];
+#pragma unroll
+            for (int j = 0; j < FINAL_BATCH; ++j) {
+                const int jj = b + j;
+                d[j] = jj < nl ? (jj < SLOTS ? cache_dev[jj * T + tid] : __ldg(pd + sub + jj * LPS)) : 0;
+                first[j] = jj < nl ? __ldg(pp + sub + jj * LPS) + e.anchor : 0u;
+            }
+#pragma unroll
+            for (int j = 0; j < FINAL_BATCH; ++j) {
+                const bool v = b + j < nl;
+                const uint32_t ir = tab_in(k, d[j] - shift) ? (uint32_t)(d[j] - shift + k.hist_base + 1) : 0u;
+                const uint32_t id = v && tab_in(k, d[j] - flen) ? (uint32_t)(d[j] - flen + k.hist_base + 1) : 0u;
+                r2[j] = D4{0, 0, 0, 0};
+                if (v) r2[j] = ld4(&k.fl[ir].l10);                                                     // log10 ref, log10p, ref, fr
+                d2[j] = D4{l10_min_prob, 0, k.min_prob, 0};                                            // floor: .b / .d unused
+                if (id) d2[j] = ld4(&k.fl[id].l10);
+            }
+            uint32_t mine = 0;                                                         // this lane's supporting read pairs, bit j
+#pragma unroll
+            for (int j = 0; j < FINAL_BATCH; ++j) {
+                const int dj = d[j];
+                if (b + j >= nl) continue;
+                mine |= (uint32_t)(dj >= delLower && dj <= delUpper) << j;
+                if (dj > upper_q) { if (dj < delLower) ++dad2; else if (dj <= delUpper) ++dad3; }
+                else { if (dj < delUpper) ++dad0; else ++dad1; }
+                const double ref = r2[j].c, del = d2[j].c;
+                if (ref >= 2 * del) ++lad0; else if (del >= 2 * ref) ++lad2;
+                t0 += r2[j].a; t2 += d2[j].a;
+                if (ref == del) { t1 += r2[j].a; ++ndeg; }                              // residue applied below
+                else if (del == k.min_prob) t1 += r2[j].b;
+                else if (ref == k.min_prob) t1 += d2[j].b;
+                else t1 += log10(ref + del) - LOG10_2_D;
+                fl_min = min(fl_min, first[j]); fl_max = max(fl_max, first[j] + (uint32_t)max(0, dj + inner_off));
+            }
+            nsp += __popc(mine);
+            const uint32_t nsup = __reduce_add_sync(PD_FULL, __popc(mine));
+            if (nsup) {
+                // one shared reservation per warp and batch (the entries' order does not matter: the percentiles bisect values)
+                uint32_t slot = 0;
+                if ((tid & 31) == 0) slot = atomicAdd(&s_nsupp, nsup);
+                slot = __shfl_sync(PD_FULL, slot, 0);
+#pragma unroll
+                for (int j = 0; j < FINAL_BATCH; ++j) {
+                    const uint32_t m = __ballot_sync(PD_FULL, (mine >> j) & 1u);
+                    if ((mine >> j) & 1u) {
+                        const uint32_t at = slot + __popc(m & lane_lt);
+                        if (at < SUPP_CAP) { s_first[at] = first[j]; s_last[at] = first[j] + (uint32_t)max(0, d[j] + inner_off); }
+                    }
+                    slot += __popc(m);
+                }
             }
         }
+        supp = nsp;
+        uint32_t lad1 = (uint32_t)nl - lad0 - lad2, dad4 = (uint32_t)nl - dad0 - dad1 - dad2 - dad3;
         lad0 = group_sum<LPS>(lad0, gmask); lad1 = group_sum<LPS>(lad1, gmask); lad2 = group_sum<LPS>(lad2, gmask);
         dad0 = group_sum<LPS>(dad0, gmask); dad1 = group_sum<LPS>(dad1, gmask); dad2 = group_sum<LPS>(dad2, gmask);
         dad3 = group_sum<LPS>(dad3, gmask); dad4 = group_sum<LPS>(dad4, gmask); ndeg = group_sum<LPS>(ndeg, gmask);
@@ -914,23 +952,21 @@ __device__ __forceinline__ void em_one_body(const PdDev & a, const EmArgs & e, E
     const unsigned long long kL = (unsigned long long)round((double)(supp - 1) * (1 - 0.8));
     uint32_t sF, sL;
     if (supp <= SUPP_CAP) {
-        if (tid < 32) {
-            const uint32_t ns = (uint32_t)supp;
-            uint32_t loF = 0xFFFFFFFFu, hiF = 0, loL = 0xFFFFFFFFu, hiL = 0;
-            for (uint32_t i = tid; i < ns; i += 32) { loF = min(loF, s_first[i]); hiF = max(hiF, s_first[i]); loL = min(loL, s_last[i]); hiL = max(hiL, s_last[i]); }
-            for (int o = 16; o > 0; o >>= 1) {
-                loF = min(loF, __shfl_xor_sync(PD_FULL, loF, o)); hiF = max(hiF, __shfl_xor_sync(PD_FULL, hiF, o));
-                loL = min(loL, __shfl_xor_sync(PD_FULL, loL, o)); hiL = max(hiL, __shfl_xor_sync(PD_FULL, hiL, o));
+        // start percentile on warp 0, end percentile on warp 1 (both on warp 0 in a one-warp block)
+        const uint32_t ns = (uint32_t)supp;
+        for (int q = tid >> 5; q < 2; q += T >> 5) {
+            const uint32_t * v = q == 0 ? s_first : s_last;
+            const unsigned long long kq = q == 0 ? kF : kL;
+            uint32_t lo = 0xFFFFFFFFu, hi = 0;
+            for (uint32_t i = tid & 31; i < ns; i += 32) { lo = min(lo, v[i]); hi = max(hi, v[i]); }
+            lo = __reduce_min_sync(PD_FULL, lo); hi = __reduce_max_sync(PD_FULL, hi);
+            while (lo < hi) {
+                const uint32_t mid = lo + (hi - lo) / 2;
+                uint32_t c = 0;
+                for (uint32_t i = tid & 31; i < ns; i += 32) c += v[i] <= mid;
+                if (__reduce_add_sync(PD_FULL, c) >= kq + 1) hi = mid; else lo = mid + 1;
             }
-            while (loF < hiF || loL < hiL) {
-                const uint32_t midF = loF + (hiF - loF) / 2, midL = loL + (hiL - loL) / 2;
-                uint32_t cF = 0, cL = 0;
-                for (uint32_t i = tid; i < ns; i += 32) { cF += s_first[i] <= midF; cL += s_last[i] <= midL; }
-                for (int o = 16; o > 0; o >>= 1) { cF += __shfl_xor_sync(PD_FULL, cF, o); cL += __shfl_xor_sync(PD_FULL, cL, o); }
-                if (loF < hiF) { if (cF >= kF + 1) hiF = midF; else loF = midF + 1; }
-                if (loL < hiL) { if (cL >= kL + 1) hiL = midL; else loL = midL + 1; }
-            }
-            if (tid == 0) { sh.sel[0] = loF; sh.sel[1] = loL; }
+            if ((tid & 31) == 0) sh.sel[q] = lo;
         }
         __syncthreads();
         sF = sh.sel[0]; sL = sh.sel[1];
@@ -939,12 +975,20 @@ __device__ __forceinline__ void em_one_body(const PdDev & a, const EmArgs & e, E
         while (loF < hiF || loL < hiL) {
             const uint32_t midF = loF + (hiF - loF) / 2, midL = loL + (hiL - loL) / 2;
             unsigned long long cF = 0, cL = 0;
-            for (int j = 0; j < nl; ++j) {
-                const int d = __ldg(pd + sub + j * LPS);
-                if (d >= delLower && d <= delUpper) {
-                    const uint32_t first = __ldg(pp + sub + j * LPS) + e.anchor;
-                    const uint32_t last = first + (uint32_t)max(0, d + inner_off);
-                    cF += first <= midF; cL += last <= midL;
+            for (int b = 0; b < nl; b += FINAL_BATCH) {
+                int d[FINAL_BATCH]; uint32_t first[FINAL_BATCH];
+#pragma unroll
+                for (int j = 0; j < FINAL_BATCH; ++j) {
+                    const int jj = b + j;
+                    d[j] = jj < nl ? (jj < SLOTS ? cache_dev[jj * T + tid] : __ldg(pd + sub + jj * LPS)) : 0;
+                    first[j] = jj < nl ? __ldg(pp + sub + jj * LPS) + e.anchor : 0u;
+                }
+#pragma unroll
+                for (int j = 0; j < FINAL_BATCH; ++j) {
+                    if (b + j < nl && d[j] >= delLower && d[j] <= delUpper) {
+                        const uint32_t last = first[j] + (uint32_t)max(0, d[j] + inner_off);
+                        cF += first[j] <= midF; cL += last <= midL;
+                    }
                 }
             }
             block_sum2u(cF, cL, sh.redu);
@@ -1153,7 +1197,9 @@ int pd_launch_em(pd_ctx * c, const PdDev & a, const EmArgs & e, cudaStream_t st,
     // Measured on B200 (100 samples x chr21, ms per step): one look-up pair in flight at 80 registers / 6 blocks per SM
     // 3.44; two in flight at 96 registers / 5 blocks 3.56; 3 / 4 in flight 3.72 / 4.02; 72 / 64 registers (7 / 8 blocks,
     // spills) 3.78 / 3.86; L1 prefetch of the table rows 5.0; two lanes per sample 5.4; EM loop and final pass as two
-    // kernels 3.56-3.76.
+    // kernels 3.56-3.76. Final pass, A/B on one B200 at 1000 W, all at 80 registers / 6 blocks: one read pair per
+    // iteration with a shared atomic per supporting pair 3.79; FINAL_BATCH = 2 read pairs per lane in flight with one
+    // reservation per warp and batch 3.68; 4 in flight 4.07 (spills inside the loop).
     if (a.R == a.N && a.N <= 256 && !getenv("PD_EM_GENERAL")) {
         const uint32_t T1 = ((a.N + 31) / 32) * 32;
         const cudaError_t err1 = T1 <= 128 ? launch_one_t<1, 32, 128, 6, 1>(a, e, T1, st) : launch_one_t<1, 32, 256, 3, 2>(a, e, T1, st);
