@@ -223,6 +223,11 @@ int pd_contig_window_count(pd_ctx * ctx, uint64_t * n_windows);
  * closed-form activity rule the kernels use. out = n_windows x 3 int64. Needs no GPU. */
 int pd_debug_host_window_sums(pd_ctx * ctx, uint32_t rg, uint64_t first_window, uint64_t n_windows, int64_t * out);
 
+/* Device-side validation hook (NOT used by the scan): the same sums as pd_debug_host_window_sums, computed on the GPU
+ * by the read-pair walk of the scan kernels over the uploaded contig (uploads it first if needed, so it works after
+ * any pd_contig_push* variant). Windows beyond the contig's tile tables are 0. out = n_windows x 3 int64 (host). */
+int pd_debug_device_window_sums(pd_ctx * ctx, uint32_t rg, uint64_t first_window, uint64_t n_windows, int64_t * out);
+
 /* Host-side validation hook for the active-coverage cap of pd_contig_push (ChromosomeProfile::add,
  * profile_structure_popdel_call.h:1084-1113): stored[i] = 1 when read pair i (anchor-relative start position and
  * end = start + max(0, inner distance), sorted by start) of a read group with cap max_load is kept. Needs no GPU. */

@@ -59,7 +59,7 @@ CALL_DTYPE = np.dtype([("initial_length", "<u4"), ("iterations", "<u4"), ("delet
 
 EXPORTS = ["pd_process_histogram", "pd_create", "pd_create_error", "pd_destroy", "pd_last_error", "pd_contig_begin",
            "pd_contig_push", "pd_contig_push_pinned", "pd_contig_push_compact", "pd_contig_push_compact32", "pd_contig_push_device", "pd_contig_upload", "pd_contig_scan", "pd_contig_window_count",
-           "pd_debug_host_window_sums", "pd_debug_cap_replay", "pd_contig_reserve_windows", "pd_shard_unique_id", "pd_shard_attach_nccl",
+           "pd_debug_host_window_sums", "pd_debug_device_window_sums", "pd_debug_cap_replay", "pd_contig_reserve_windows", "pd_shard_unique_id", "pd_shard_attach_nccl",
            "pd_shard_attach_group", "pd_shard_group_scan", "pd_set_unify", "pd_device_warmup", "pd_set_staging"]
 
 _lib = None
@@ -99,6 +99,7 @@ def load_library(path: str = LIB_PATH):
     lib.pd_contig_scan.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.POINTER(PdResult)]
     lib.pd_contig_window_count.argtypes = [C.c_void_p, C.POINTER(C.c_uint64)]
     lib.pd_debug_host_window_sums.argtypes = [C.c_void_p, C.c_uint32, C.c_uint64, C.c_uint64, C.POINTER(C.c_int64)]
+    lib.pd_debug_device_window_sums.argtypes = lib.pd_debug_host_window_sums.argtypes
     lib.pd_contig_reserve_windows.argtypes = [C.c_void_p, C.c_uint64]
     lib.pd_shard_unique_id.argtypes = [C.POINTER(C.c_uint8)]
     lib.pd_shard_attach_nccl.argtypes = [C.c_void_p, C.POINTER(PdShardInfo), C.POINTER(C.c_uint8)]
@@ -374,6 +375,14 @@ class Scanner:
                                                        out.ctypes.data_as(C.POINTER(C.c_int64))))
         return out
 
+    def debug_device_window_sums(self, rg: int, first_window: int, n_windows: int) -> np.ndarray:
+        """pd_debug_device_window_sums: the sums of debug_host_window_sums, taken by the scan kernels' read-pair walk over
+        the uploaded contig (uploads it first)."""
+        out = np.zeros((int(n_windows), 3), dtype=np.int64)
+        self._check(self.lib.pd_debug_device_window_sums(self.ctx, int(rg), int(first_window), int(n_windows),
+                                                         out.ctypes.data_as(C.POINTER(C.c_int64))))
+        return out
+
 
 def synth_read_group(seed: int, rg_index: int, mu: float, sigma: float, read_length: int, pairs_per_bp: float,
                      first_pos: int, end_pos: int, del_start=(), del_len=(), del_genotype=()):
@@ -518,30 +527,38 @@ def scan_cohort(samples, params: CallParameters, device: int = 0, first_window: 
     try:
         if unify:
             sc.set_unify(**unify)
-        sc.begin_contig(cohort_anchor(samples))
-        g = 0
-        keep = []
-        for s in samples:
-            for rg in s.read_groups:
-                if pinned == "device":                          # arrays already resident on the GPU (pd_contig_push_device)
-                    import torch
-                    dp = torch.from_numpy(np.ascontiguousarray(rg.pos, dtype=np.uint32).view(np.int32)).to(f"cuda:{device}")
-                    dd = torch.from_numpy(np.ascontiguousarray(rg.dev, dtype=np.int32)).to(f"cuda:{device}")
-                    keep.append((dp, dd))
-                    sc.push_device(g, dp.numel(), dp.data_ptr(), dd.data_ptr())
-                elif pinned == "compact32":
-                    sc.push_compact32(g, *[_page_locked(a) for a in compact32_encode(rg.pos, rg.dev)])
-                elif pinned == "compact":
-                    sc.push_compact(g, *[_page_locked(a) for a in compact_encode(rg.pos, rg.dev)])
-                elif pinned:
-                    sc.push_pinned(g, _page_locked(np.ascontiguousarray(rg.pos, dtype=np.uint32)),
-                                   _page_locked(np.ascontiguousarray(rg.dev, dtype=np.int32)))
-                else:
-                    sc.push(g, rg.pos, rg.dev)
-                g += 1
+        keep = push_cohort(sc, samples, pinned, device)      # (device arrays must outlive the scan)
         return sc.scan(first_window, n_windows), rgs
     finally:
         sc.close()
+
+
+def push_cohort(sc: Scanner, samples, pinned=False, device: int = 0) -> list:
+    """Opens the contig of an in-memory cohort on `sc` and pushes every read group with one of the push variants:
+    False = pd_contig_push, True = _pinned, "compact", "compact32", "device". Returns the device arrays of the "device"
+    variant, which must stay alive until the upload."""
+    sc.begin_contig(cohort_anchor(samples))
+    g = 0
+    keep = []
+    for s in samples:
+        for rg in s.read_groups:
+            if pinned == "device":                          # arrays already resident on the GPU (pd_contig_push_device)
+                import torch
+                dp = torch.from_numpy(np.ascontiguousarray(rg.pos, dtype=np.uint32).view(np.int32)).to(f"cuda:{device}")
+                dd = torch.from_numpy(np.ascontiguousarray(rg.dev, dtype=np.int32)).to(f"cuda:{device}")
+                keep.append((dp, dd))
+                sc.push_device(g, dp.numel(), dp.data_ptr(), dd.data_ptr())
+            elif pinned == "compact32":
+                sc.push_compact32(g, *[_page_locked(a) for a in compact32_encode(rg.pos, rg.dev)])
+            elif pinned == "compact":
+                sc.push_compact(g, *[_page_locked(a) for a in compact_encode(rg.pos, rg.dev)])
+            elif pinned:
+                sc.push_pinned(g, _page_locked(np.ascontiguousarray(rg.pos, dtype=np.uint32)),
+                               _page_locked(np.ascontiguousarray(rg.dev, dtype=np.int32)))
+            else:
+                sc.push(g, rg.pos, rg.dev)
+            g += 1
+    return keep
 
 
 def shard_unique_id() -> bytes:

@@ -53,6 +53,10 @@ void pd_launch_gran_index(const PdDev & a, uint32_t * gran_tile, const uint32_t 
 void pd_launch_tile_segs(uint4 * out, uint32_t n, uint32_t window_buffer, cudaStream_t st);
 void pd_launch_screen(const PdDev & a, const ScreenArgs & s, uint32_t max_rg_words, cudaStream_t st, cudaEvent_t after_stream, uint64_t * launches);
 void pd_launch_tile_jobs(const JobArgs & j, cudaStream_t st, uint64_t * launches);
+// pd_debug_device_window_sums: per-window count / sum of deviations / sum of positions of read group g, windows [w_first, w_end)
+// of tiles [tile_begin, tile_end), as for_tile_batches walks them; out[3 * (w - w_first) + k]
+void pd_launch_window_sums(const PdDev & a, uint32_t g, uint32_t anchor, uint32_t tile_begin, uint32_t tile_end, uint64_t w_first,
+                           uint64_t w_end, unsigned long long * out, cudaStream_t st);
 
 // ---- gather + candidates (pd_gather.cu) -----------------------------------------------------------------------
 struct GatherArgs {

@@ -89,6 +89,17 @@ int build_index(pd_ctx * c, PdDev & a)
     return 0;
 }
 
+// device view of the uploaded contig (the window range and thresholds are the caller's); builds the index once per upload
+int device_view(pd_ctx * c, PdDev & a)
+{
+    a = PdDev{};
+    a.words = c->d_words; a.tiles = c->d_tiles; a.longs = c->d_longs;
+    a.rgc = c->d_rgc; a.sample_rg = c->d_sample_rg; a.tab = c->d_tab;
+    a.NT = c->NT; a.N = c->N; a.R = c->R; a.window_buffer = c->grid.window_buffer; a.t_min = c->t_min;
+    a.tseg = c->d_tseg;
+    return c->index_built ? 0 : build_index(c, a);
+}
+
 // mapped, page-locked result buffers: grown so that `need_calls` calls fit; existing contents are preserved
 int ensure_results(pd_ctx * c, size_t need_calls, size_t row, size_t keep_calls)
 {
@@ -150,9 +161,7 @@ int pd_run_scan(pd_ctx * c, uint64_t first_window, uint64_t n_windows, pd_result
     out->n_windows = W;
 
     PdDev a;
-    a.words = c->d_words; a.tiles = c->d_tiles; a.longs = c->d_longs;
-    a.rgc = c->d_rgc; a.sample_rg = c->d_sample_rg; a.tab = c->d_tab;
-    a.NT = c->NT; a.N = N; a.R = R; a.window_buffer = c->grid.window_buffer; a.t_min = c->t_min;
+    if (device_view(c, a)) return c->status;
     // Second screen stage (pd_gather.cu, k_screen2): worth it when the read groups have different initial-length thresholds,
     // i.e. when the cohort-minimum threshold t_min lets nearly every window through the first stage. PD_SCREEN2=0/1 overrides.
     bool screen2 = false;
@@ -166,8 +175,6 @@ int pd_run_scan(pd_ctx * c, uint64_t first_window, uint64_t n_windows, pd_result
     a.t_known = screen2 ? std::max(c->t_min - s2gap, c->t_min / 2) : 0;
     a.t_mark = screen2 ? a.t_known : a.t_min;
     a.w_begin = (uint32_t)w_begin; a.w_end = (uint32_t)w_end;
-    a.tseg = c->d_tseg;
-    if (!c->index_built && build_index(c, a)) return c->status;
 
     cudaStream_t st = c->stream, st2 = c->stream2;
     uint64_t * nl = &out->n_kernel_launches;
@@ -533,5 +540,37 @@ int pd_run_scan(pd_ctx * c, uint64_t first_window, uint64_t n_windows, pd_result
     PD_CUDA(c, cudaEventElapsedTime(&out->ms_genotype, c->ev[4], c->ev[5]));
     PD_CUDA(c, cudaEventElapsedTime(&out->ms_total, c->ev[2], c->ev[5]));
     out->ms_d2h = 0;
+    return 0;
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// device-side validation hook: per-window sums of one read group as the scan kernels' read-pair walk sees them
+// ---------------------------------------------------------------------------------------------------------
+extern "C" int pd_debug_device_window_sums(pd_ctx * c, uint32_t rg, uint64_t first_window, uint64_t n_windows, int64_t * out)
+{
+    if (!c || !out || rg >= c->R) return PD_ERR_ARG;
+    if (c->status) return c->status;
+    if (c->device < 0) return pd_fail(c, PD_ERR_CUDA, "pd_debug_device_window_sums: host-only context (device = -1)");
+    if (!c->contig_open) return pd_fail(c, PD_ERR_ARG, "no open contig");
+    if (!c->uploaded) { const int rc = pd_contig_upload(c); if (rc) return rc; }
+    PD_CUDA(c, cudaSetDevice(c->device));
+    PdDev a;
+    if (device_view(c, a)) return c->status;
+    memset(out, 0, sizeof(int64_t) * 3 * n_windows);
+    const uint64_t t0 = first_window / PD_TILE_WINDOWS;
+    const uint64_t t1 = std::min<uint64_t>((first_window + n_windows + PD_TILE_WINDOWS - 1) / PD_TILE_WINDOWS, c->NT);
+    if (n_windows == 0 || t0 >= t1) return 0;
+    unsigned long long * d_out = nullptr;
+    const size_t bytes = sizeof(unsigned long long) * 3 * n_windows;
+    PD_CUDA(c, cudaMalloc(&d_out, bytes));
+    cudaError_t e = cudaMemsetAsync(d_out, 0, bytes, c->stream);
+    if (e == cudaSuccess) {
+        pd_launch_window_sums(a, rg, c->grid.anchor, (uint32_t)t0, (uint32_t)t1, first_window, first_window + n_windows, d_out, c->stream);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out, d_out, bytes, cudaMemcpyDeviceToHost, c->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+    cudaFree(d_out);
+    if (e != cudaSuccess) return pd_fail(c, PD_ERR_CUDA, std::string("pd_debug_device_window_sums: ") + cudaGetErrorString(e));
     return 0;
 }

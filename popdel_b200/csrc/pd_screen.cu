@@ -196,6 +196,41 @@ __global__ void __launch_bounds__(256) k_count(PdDev a, ScreenArgs s)
 }
 
 // ------------------------------------------------------------------------------------------------------------------
+// pd_debug_device_window_sums: one warp per tile of read group g. Every read pair that for_tile_batches hands out and
+// that is active in a window of [w_first, w_end) inside the tile adds its count, deviation and position to that window.
+// ------------------------------------------------------------------------------------------------------------------
+constexpr int WS_WARPS = 4;
+
+__global__ void __launch_bounds__(WS_WARPS * 32) k_window_sums(PdDev a, uint32_t g, uint32_t anchor, uint32_t tile_begin, uint32_t tile_end,
+                                                               uint64_t w_first, uint64_t w_end, unsigned long long * __restrict__ out)
+{
+    __shared__ unsigned long long sums[WS_WARPS][PD_TILE_WINDOWS * 3];
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    const uint32_t tile = tile_begin + blockIdx.x * WS_WARPS + wib;
+    if (tile >= tile_end) return;                                   // warp-uniform
+    unsigned long long * sm = sums[wib];
+    for (int i = lane; i < (int)PD_TILE_WINDOWS * 3; i += 32) sm[i] = 0;
+    __syncwarp();
+    const PdRgConst k = a.rgc[g];
+    const int64_t w0 = (int64_t)tile * PD_TILE_WINDOWS;
+    const int64_t lo = max(w0, (int64_t)w_first), hi = min(w0 + (int64_t)PD_TILE_WINDOWS - 1, (int64_t)w_end - 1);
+    for_tile_batches(a, g, k, tile, lane, [&](bool valid, int32_t s, int32_t e, uint32_t pr, int32_t dev) {
+        if (!valid) return;
+        for (int64_t w = max((int64_t)s, lo); w <= min((int64_t)e, hi); ++w) {
+            unsigned long long * o = sm + 3 * (w - w0);
+            atomicAdd(o, 1ull);
+            atomicAdd(o + 1, (unsigned long long)(long long)dev);
+            atomicAdd(o + 2, (unsigned long long)pr + anchor);
+        }
+    });
+    __syncwarp();
+    for (int i = lane; i < (int)PD_TILE_WINDOWS * 3; i += 32) {
+        const int64_t w = w0 + i / 3;
+        if (w >= lo && w <= hi) out[3 * (w - (int64_t)w_first) + i % 3] = sm[i];
+    }
+}
+
+// ------------------------------------------------------------------------------------------------------------------
 // tile jobs: flagged tiles in ascending order with their window masks; window jobs numbered in ascending order
 // ------------------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ unsigned long long tj_value(const JobArgs & j, uint32_t t, uint32_t & mask)
@@ -279,4 +314,10 @@ void pd_launch_tile_jobs(const JobArgs & j, cudaStream_t st, uint64_t * launches
     k_tj_offsets<<<1, 1024, 0, st>>>(j, nb);
     k_tj_write<<<nb, 1024, 0, st>>>(j);
     *launches += 3;
+}
+
+void pd_launch_window_sums(const PdDev & a, uint32_t g, uint32_t anchor, uint32_t tile_begin, uint32_t tile_end, uint64_t w_first,
+                           uint64_t w_end, unsigned long long * out, cudaStream_t st)
+{
+    k_window_sums<<<(tile_end - tile_begin + WS_WARPS - 1) / WS_WARPS, WS_WARPS * 32, 0, st>>>(a, g, anchor, tile_begin, tile_end, w_first, w_end, out);
 }

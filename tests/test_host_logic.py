@@ -139,10 +139,75 @@ def _cohort(kind):
         # a large deletion (long read pairs in the wide list) crossing a segment border
         dels = [simulate.Deletion(196_000, 9000, np.array([1, 2, 1]))]
         return simulate.simulate_cohort(seed=26, n_samples=3, contig_len=260_000, n_dels=0, dels=dels)[0], api.CallParameters()
+    if kind in _LIBRARY_KINDS:
+        return _library_cohort(kind), api.CallParameters()
     raise KeyError(kind)
 
 
-@pytest.mark.parametrize("kind", ["basic", "mixedrg", "gap", "highcov", "longspan", "capborder", "capgap", "capspill", "capfar"])
+# Libraries other than ~500 +- 80 bp / 150-bp reads. The insert-size distribution decides the look-back of the packed
+# stream (pd_create: ceil(((29 + median - 2 readLen + 8 sd) / 30 + 2) / 32) tiles, at most PD_MAX_LOOKBACK_TILES = 8),
+# how many read pairs go to the wide list and how many rows the likelihood tables have (hist_end - hist_start):
+#   wideins   900 +- 150, 100-bp reads: look-back 3
+#   matepair  2 500 +- 400: look-back 6, a 20-kbp hole in one sample (tiles without read pairs inside the look-back),
+#             2 401-row tables (the sample-major EM with more than 48 KB of dynamic shared memory)
+#   longins   8 000 +- 1 200: look-back clamped at 8, most read pairs in the wide list, 7 201-row tables (sample-major EM off)
+#   overlap   330 +- 60 at 50x with a quarter of the insert sizes in [0, 300): overlapping reads, inner distance clamped to 0,
+#             deviations down to -median
+#   megadel   a 1.1-Mbp deletion: deviations above PD_DEV_MAX (clamped in the stream word, kept in the wide list) and Q3
+#             values beyond the presence bitmap of the candidate step
+#   manyrg    10 read groups per sample with mixed read lengths: more read groups than the gather's fast path holds
+_LIBRARY_KINDS = ("wideins", "matepair", "longins", "overlap", "megadel", "manyrg")
+
+
+def _library_cohort(kind):
+    spec = simulate.ReadGroupSpec
+
+    def genotypes(n, p):
+        return np.random.default_rng(5).binomial(2, p, size=n)
+
+    if kind == "wideins":
+        specs = [[spec(name=f"rg{s}", mu=900, sigma=150, read_length=100, coverage=20)] for s in range(6)]
+        dels = [simulate.Deletion(100_000, 2500, genotypes(6, 0.5))]
+        return simulate.simulate_cohort(seed=51, n_samples=6, contig_len=200_000, n_dels=0, dels=dels, rg_specs=specs)[0]
+    if kind == "matepair":
+        specs = [[spec(name=f"rg{s}", mu=2500, sigma=400, coverage=8)] for s in range(6)]
+        dels = [simulate.Deletion(100_000, 5000, genotypes(6, 0.5))]
+        samples = simulate.simulate_cohort(seed=51, n_samples=6, contig_len=200_000, n_dels=0, dels=dels, rg_specs=specs)[0]
+        rg = samples[2].read_groups[0]
+        keep = ~((rg.pos >= 40_000) & (rg.pos < 60_000))
+        rg.pos, rg.isize = rg.pos[keep], rg.isize[keep]
+        return samples
+    if kind == "longins":
+        specs = [[spec(name=f"rg{s}", mu=8000, sigma=1200, coverage=3)] for s in range(6)]
+        dels = [simulate.Deletion(130_000, 9000, genotypes(6, 0.5))]
+        return simulate.simulate_cohort(seed=51, n_samples=6, contig_len=260_000, n_dels=0, dels=dels, rg_specs=specs)[0]
+    if kind == "overlap":
+        # 50x: at 30x a hom carrier keeps a single active read pair right after the deletion, and its reference shift is
+        # the x87 artefact of DESIGN 2 (the shift quotient lands on the deviation or one ulp below it)
+        specs = [[spec(name=f"rg{s}", mu=330, sigma=60, coverage=50)] for s in range(4)]
+        dels = [simulate.Deletion(60_000, 800, genotypes(4, 0.5))]
+        samples = simulate.simulate_cohort(seed=51, n_samples=4, contig_len=120_000, n_dels=0, dels=dels, rg_specs=specs)[0]
+        rng = np.random.default_rng(52)
+        for s in samples:
+            rg = s.read_groups[0]
+            short = rng.random(rg.pos.size) < 0.25              # the simulator clips insert sizes at 2 * readLen
+            isz = np.where(short, rng.integers(0, 300, size=rg.pos.size), rg.isize).astype(np.int32)
+            o = np.lexsort((isz, rg.pos))
+            rg.pos, rg.isize = rg.pos[o], isz[o]
+            simulate.finalize_histogram(rg)
+        return samples
+    if kind == "megadel":
+        dels = [simulate.Deletion(200_000, 1_100_000, genotypes(4, 0.5))]
+        return simulate.simulate_cohort(seed=51, n_samples=4, contig_len=1_500_000, n_dels=0, dels=dels)[0]
+    if kind == "manyrg":
+        specs = [[spec(name=f"s{s}_rg{j}", mu=(350, 450, 550)[j % 3], sigma=(30, 50, 80)[(j + s) % 3],
+                       read_length=(100, 125, 150)[(j // 3 + s) % 3], coverage=15) for j in range(10)] for s in range(3)]
+        return simulate.simulate_cohort(seed=51, n_samples=3, contig_len=150_000, n_dels=2, rg_specs=specs)[0]
+    raise KeyError(kind)
+
+
+@pytest.mark.parametrize("kind", ["basic", "mixedrg", "gap", "highcov", "longspan", "capborder", "capgap", "capspill", "capfar",
+                                  "wideins", "matepair", "longins", "overlap", "megadel", "manyrg"])
 def test_packed_layout_reproduces_active_sets(kind, oracle_lib):
     from parity import run_oracle
     samples, params = _cohort(kind)
@@ -235,6 +300,8 @@ def test_error_behaviour_of_the_c_abi_without_a_gpu():
     sc3.push(0, rg.pos, rg.dev)
     sc3.reserve_windows(5000)
     assert sc3.window_count() > 1000
+    with pytest.raises(api.ScanError, match="window_sums: host-only context"):
+        sc3.debug_device_window_sums(0, 0, 100)                                # the device probe has no CPU path either
     with pytest.raises(api.ScanError, match="host-only context"):
         sc3.scan()
     with pytest.raises(api.ScanError, match="no usable CUDA device|out of range"):

@@ -11,7 +11,8 @@ from test_host_logic import _cohort
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.parametrize("kind", ["basic", "mixedrg", "gap", "highcov", "longspan", "capspill", "capfar"])
+@pytest.mark.parametrize("kind", ["basic", "mixedrg", "gap", "highcov", "longspan", "capspill", "capfar",
+                                  "wideins", "matepair", "longins", "overlap", "megadel", "manyrg"])
 def test_scan_matches_oracle(kind, oracle_lib):
     samples, params = _cohort(kind)
     stats = compare_scan_with_oracle(samples, oracle_lib, params)
@@ -69,7 +70,8 @@ def test_larger_cohort(oracle_lib):
     assert stats["n_calls"] > 100
 
 
-@pytest.mark.parametrize("kind", ["basic", "mixedrg", "gap", "highcov", "longspan", "capspill", "capfar"])
+@pytest.mark.parametrize("kind", ["basic", "mixedrg", "gap", "highcov", "longspan", "capspill", "capfar",
+                                  "wideins", "matepair", "longins", "overlap", "megadel", "manyrg"])
 def test_device_packer_equals_host_packer(kind):
     """pd_contig_push_pinned / _compact / _device (device-side packing; host fallback when the coverage cap bites) == pd_contig_push."""
     samples, params = _cohort(kind)
@@ -141,7 +143,7 @@ def test_many_samples(n_samples, contig_len, env, oracle_lib, monkeypatch):
 @pytest.mark.parametrize("env", [{"PD_FORCE_SLOW": "7"}, {"PD_JOB_BATCH": "64", "PD_CJOB_ROWS": "7"}, {"PD_CJOB_ROWS": "1", "PD_EM_CHUNK": "5"},
                                  {"PD_EM_GENERAL": "1"}, {"PD_EM_V2": "1"}, {"PD_EM_V1": "1"}, {"PD_SCREEN2": "1"}, {"PD_SCREEN2": "0"},
                                  {"PD_SCREEN2": "1", "PD_FORCE_SLOW": "7", "PD_JOB_BATCH": "64"}])
-@pytest.mark.parametrize("kind", ["basic", "mixedrg", "highcov"])
+@pytest.mark.parametrize("kind", ["basic", "mixedrg", "highcov", "matepair", "longins", "megadel"])
 def test_scan_generic_paths_and_batching(kind, env, oracle_lib, monkeypatch):
     """The generic (no shared memory) Q3 / pool paths, small job batches, candidate-job sub-batches and EM chunks, and
     the general EM kernel give the same calls as the default configuration (all knobs are read per scan)."""
@@ -151,7 +153,7 @@ def test_scan_generic_paths_and_batching(kind, env, oracle_lib, monkeypatch):
     compare_scan_with_oracle(samples, oracle_lib, params)
 
 
-@pytest.mark.parametrize("kind,world", [("basic", 2), ("mixedrg", 2), ("mixedrg", 3), ("highcov", 2), ("longspan", 3)])
+@pytest.mark.parametrize("kind,world", [("basic", 2), ("mixedrg", 2), ("mixedrg", 3), ("highcov", 2), ("longspan", 3), ("matepair", 2)])
 def test_sample_sharded_scan_equals_single_context(kind, world, oracle_lib):
     """Sample sharding (SURVEY.md 8e, config 5): `world` contexts of one process, each holding a block of the samples,
     exchange tile flags, Q3 values and the EM's per-iteration statistics (in-kernel, through peer memory). The merged
