@@ -228,6 +228,14 @@ int pd_debug_host_window_sums(pd_ctx * ctx, uint32_t rg, uint64_t first_window, 
  * any pd_contig_push* variant). Windows beyond the contig's tile tables are 0. out = n_windows x 3 int64 (host). */
 int pd_debug_device_window_sums(pd_ctx * ctx, uint32_t rg, uint64_t first_window, uint64_t n_windows, int64_t * out);
 
+/* Device-side validation hook (NOT used by the scan): runs the device-side unifyCalls of pd_set_unify on n caller-built
+ * window calls instead of a scan's. calls[n] are in window order with segment tags < nseg (a segment's calls are one run
+ * of equal tags), per_sample holds their n x n_samples x 13 rows (host memory). They are copied to the device buffers a
+ * scan leaves its window calls in and merged by the same kernels with the context's pd_set_unify settings; `out` receives
+ * the merged variants, their rows and significant windows as after pd_contig_scan. Refuses (PD_ERR_ARG) a context without
+ * pd_set_unify, a host-only context and a sample-sharded one. Needs no contig. */
+int pd_debug_unify(pd_ctx * ctx, uint64_t n, const pd_call * calls, const uint32_t * per_sample, uint32_t nseg, pd_result * out);
+
 /* Host-side validation hook for the active-coverage cap of pd_contig_push (ChromosomeProfile::add,
  * profile_structure_popdel_call.h:1084-1113): stored[i] = 1 when read pair i (anchor-relative start position and
  * end = start + max(0, inner distance), sorted by start) of a read group with cap max_load is kept. Needs no GPU. */

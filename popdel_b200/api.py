@@ -59,7 +59,7 @@ CALL_DTYPE = np.dtype([("initial_length", "<u4"), ("iterations", "<u4"), ("delet
 
 EXPORTS = ["pd_process_histogram", "pd_create", "pd_create_error", "pd_destroy", "pd_last_error", "pd_contig_begin",
            "pd_contig_push", "pd_contig_push_pinned", "pd_contig_push_compact", "pd_contig_push_compact32", "pd_contig_push_device", "pd_contig_upload", "pd_contig_scan", "pd_contig_window_count",
-           "pd_debug_host_window_sums", "pd_debug_device_window_sums", "pd_debug_cap_replay", "pd_contig_reserve_windows", "pd_shard_unique_id", "pd_shard_attach_nccl",
+           "pd_debug_host_window_sums", "pd_debug_device_window_sums", "pd_debug_unify", "pd_debug_cap_replay", "pd_contig_reserve_windows", "pd_shard_unique_id", "pd_shard_attach_nccl",
            "pd_shard_attach_group", "pd_shard_group_scan", "pd_set_unify", "pd_device_warmup", "pd_set_staging"]
 
 _lib = None
@@ -100,6 +100,7 @@ def load_library(path: str = LIB_PATH):
     lib.pd_contig_window_count.argtypes = [C.c_void_p, C.POINTER(C.c_uint64)]
     lib.pd_debug_host_window_sums.argtypes = [C.c_void_p, C.c_uint32, C.c_uint64, C.c_uint64, C.POINTER(C.c_int64)]
     lib.pd_debug_device_window_sums.argtypes = lib.pd_debug_host_window_sums.argtypes
+    lib.pd_debug_unify.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.POINTER(C.c_uint32), C.c_uint32, C.POINTER(PdResult)]
     lib.pd_contig_reserve_windows.argtypes = [C.c_void_p, C.c_uint64]
     lib.pd_shard_unique_id.argtypes = [C.POINTER(C.c_uint8)]
     lib.pd_shard_attach_nccl.argtypes = [C.c_void_p, C.POINTER(PdShardInfo), C.POINTER(C.c_uint8)]
@@ -381,6 +382,21 @@ class Scanner:
         out = np.zeros((int(n_windows), 3), dtype=np.int64)
         self._check(self.lib.pd_debug_device_window_sums(self.ctx, int(rg), int(first_window), int(n_windows),
                                                          out.ctypes.data_as(C.POINTER(C.c_int64))))
+        return out
+
+    def debug_unify(self, calls: np.ndarray, per_sample: np.ndarray, nseg: int) -> dict:
+        """pd_debug_unify: the device-side merge of set_unify on caller-built window calls (CALL_DTYPE records in window
+        order, segment tags < nseg) and their per-sample rows [n, n_samples, 13]. Returns what scan() returns in unify
+        mode (`significant_windows` is an empty array when there is no variant)."""
+        calls = np.ascontiguousarray(calls, dtype=CALL_DTYPE)
+        per = np.ascontiguousarray(per_sample, dtype=np.uint32)
+        assert per.shape == (calls.size, self.n_samples, 13)
+        res = PdResult()
+        self._check(self.lib.pd_debug_unify(self.ctx, calls.size, calls.ctypes.data_as(C.c_void_p),
+                                            per.ctypes.data_as(C.POINTER(C.c_uint32)), int(nseg), C.byref(res)))
+        out = self._result_dict(res)
+        if out["significant_windows"] is None:
+            out["significant_windows"] = np.zeros(0, dtype=np.uint32)
         return out
 
 

@@ -574,3 +574,35 @@ extern "C" int pd_debug_device_window_sums(pd_ctx * c, uint32_t rg, uint64_t fir
     if (e != cudaSuccess) return pd_fail(c, PD_ERR_CUDA, std::string("pd_debug_device_window_sums: ") + cudaGetErrorString(e));
     return 0;
 }
+
+// ---------------------------------------------------------------------------------------------------------
+// device-side validation hook: the segment-level merge (pd_run_unify) of caller-built window calls
+// ---------------------------------------------------------------------------------------------------------
+extern "C" int pd_debug_unify(pd_ctx * c, uint64_t n, const pd_call * calls, const uint32_t * per_sample, uint32_t nseg, pd_result * out)
+{
+    if (!c || !out || (n && (!calls || !per_sample))) return PD_ERR_ARG;
+    if (c->status) return c->status;
+    if (c->device < 0) return pd_fail(c, PD_ERR_ARG, "pd_debug_unify: host-only context (device = -1)");
+    if (!c->unify_on) return pd_fail(c, PD_ERR_ARG, "pd_debug_unify: no unify settings (call pd_set_unify first)");
+    if (c->shard) return pd_fail(c, PD_ERR_ARG, "pd_debug_unify: sample-sharded context (the probe merges one context's calls)");
+    if (n > 0xFFFFFFFFull) return pd_fail(c, PD_ERR_ARG, "pd_debug_unify: more than 2^32 - 1 window calls");
+    for (uint64_t i = 0; i < n; ++i)      // the merge takes a segment's calls as one run of equal tags (k_seg_bounds)
+        if (calls[i].segment >= nseg || (i && calls[i].segment < calls[i - 1].segment))
+            return pd_fail(c, PD_ERR_ARG, "pd_debug_unify: segment tags must be < nseg and in ascending order");
+    PD_CUDA(c, cudaSetDevice(c->device));
+    memset(out, 0, sizeof(*out));
+    const size_t row = 13ull * c->N;
+    if (ensure_results(c, 1, row, 0)) return c->status;
+    if (pd_unify_ensure_raw(c, std::max<uint64_t>(n, 1), row, 0)) return c->status;
+    if (n) {
+        PD_CUDA(c, cudaMemcpyAsync(c->d_u_calls, calls, n * sizeof(pd_call), cudaMemcpyHostToDevice, c->stream));
+        PD_CUDA(c, cudaMemcpyAsync(c->d_u_ps, per_sample, n * row * 4, cudaMemcpyHostToDevice, c->stream));
+    }
+    out->n_window_calls = n;
+    if (pd_run_unify(c, (uint32_t)n, row, nseg, ensure_results, &out->n_calls, &out->n_kernel_launches)) return c->status;
+    PD_CUDA(c, cudaStreamSynchronize(c->stream));
+    out->calls = c->res_calls;
+    out->per_sample = c->res_ps;
+    out->significant_windows = c->res_sig;
+    return 0;
+}

@@ -304,6 +304,11 @@ def test_error_behaviour_of_the_c_abi_without_a_gpu():
         sc3.debug_device_window_sums(0, 0, 100)                                # the device probe has no CPU path either
     with pytest.raises(api.ScanError, match="host-only context"):
         sc3.scan()
+    sc4, _ = _tiny_scanner(device=-1)
+    sc4.set_unify(50.0, 0.5, False)
+    calls = np.zeros(2, dtype=api.CALL_DTYPE)
+    with pytest.raises(api.ScanError, match=r"^\[-1\] pd_debug_unify: host-only context"):
+        sc4.debug_unify(calls, np.zeros((2, 2, 13), np.uint32), 1)              # the merge probe has no CPU path: PD_ERR_ARG
     with pytest.raises(api.ScanError, match="no usable CUDA device|out of range"):
         _tiny_scanner(device=99)
 

@@ -205,10 +205,13 @@ def _mean_stddev(rgs):
 
 
 @pytest.mark.parametrize("output_failed", [False, True])
-@pytest.mark.parametrize("kind", ["basic", "mixedrg", "gap", "highcov", "longspan"])
+@pytest.mark.parametrize("kind", ["basic", "mixedrg", "gap", "highcov", "longspan", "capspill", "capfar",
+                                  "wideins", "matepair", "longins", "overlap", "megadel", "manyrg"])
 def test_device_unify_equals_oracle_unify(kind, output_failed, oracle_lib):
     """pd_set_unify (unifyCalls on the device, SURVEY.md 8f rank 1): the merged variants equal the oracle's unifyCalls
-    (utils_popdel.h:567-654, pinned against the reference's merged VCFs) applied to the same window calls."""
+    (utils_popdel.h:567-654, pinned against the reference's merged VCFs) applied to the same window calls. matepair,
+    longins and megadel have segments of 973 to 8 446 window calls (past the merge loop's 512 shared-memory slots) and
+    variants with more than 1 024 in-range windows (past the values a warp stages for the median)."""
     samples, params = _cohort(kind)
     raw, rgs = api.scan_cohort(samples, params)
     sd = _mean_stddev(rgs)

@@ -13,8 +13,10 @@ from test_host_logic import _cohort
 
 pytestmark = pytest.mark.gpu
 
-# (highcov has two samples: a third rank would hold none)
-KIND_WORLD = [(k, w) for k in ["basic", "mixedrg", "gap", "highcov", "longspan"] for w in (2, 3) if (k, w) != ("highcov", 3)]
+# (highcov has two samples: a third rank would hold none; matepair, longins and megadel: segments past the merge loop's
+# shared-memory slots and variants past the median's staged values)
+KIND_WORLD = [(k, w) for k in ["basic", "mixedrg", "gap", "highcov", "longspan"] for w in (2, 3) if (k, w) != ("highcov", 3)] + \
+    [("matepair", 2), ("longins", 2), ("megadel", 2)]
 
 
 def _mean_stddev(rgs):
