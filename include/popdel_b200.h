@@ -236,6 +236,16 @@ int pd_debug_device_window_sums(pd_ctx * ctx, uint32_t rg, uint64_t first_window
  * pd_set_unify, a host-only context and a sample-sharded one. Needs no contig. */
 int pd_debug_unify(pd_ctx * ctx, uint64_t n, const pd_call * calls, const uint32_t * per_sample, uint32_t nseg, pd_result * out);
 
+/* Device-side validation hook (NOT used by the scan): initialize_deletion_lengths (genotype_deletion_popdel_call.h:58-86)
+ * of n_windows caller-built windows, run by the scan's candidate step with the context's rank-indexed thresholds
+ * (min_init_del_len of read groups 0, 1, ... in the order of the sorted Q3s) and the same choice of kernel instance.
+ * q3 and state are [n_windows][n_samples] host arrays; a sample takes part where its state byte is 2 ("has a Q3").
+ * counts[n_windows] receives each window's number of candidate lengths, cands the lengths of all windows in window order,
+ * ascending within a window, at most `cap` of them (PD_ERR_CAPACITY when there are more). Refuses (PD_ERR_ARG) a
+ * host-only and a sample-sharded context. Needs no contig. */
+int pd_debug_candidates(pd_ctx * ctx, uint64_t n_windows, const int32_t * q3, const uint8_t * state, uint32_t * counts,
+                        int32_t * cands, uint64_t cap);
+
 /* Host-side validation hook for the active-coverage cap of pd_contig_push (ChromosomeProfile::add,
  * profile_structure_popdel_call.h:1084-1113): stored[i] = 1 when read pair i (anchor-relative start position and
  * end = start + max(0, inner distance), sorted by start) of a read group with cap max_load is kept. Needs no GPU. */

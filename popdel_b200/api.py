@@ -59,7 +59,7 @@ CALL_DTYPE = np.dtype([("initial_length", "<u4"), ("iterations", "<u4"), ("delet
 
 EXPORTS = ["pd_process_histogram", "pd_create", "pd_create_error", "pd_destroy", "pd_last_error", "pd_contig_begin",
            "pd_contig_push", "pd_contig_push_pinned", "pd_contig_push_compact", "pd_contig_push_compact32", "pd_contig_push_device", "pd_contig_upload", "pd_contig_scan", "pd_contig_window_count",
-           "pd_debug_host_window_sums", "pd_debug_device_window_sums", "pd_debug_unify", "pd_debug_cap_replay", "pd_contig_reserve_windows", "pd_shard_unique_id", "pd_shard_attach_nccl",
+           "pd_debug_host_window_sums", "pd_debug_device_window_sums", "pd_debug_unify", "pd_debug_candidates", "pd_debug_cap_replay", "pd_contig_reserve_windows", "pd_shard_unique_id", "pd_shard_attach_nccl",
            "pd_shard_attach_group", "pd_shard_group_scan", "pd_set_unify", "pd_device_warmup", "pd_set_staging"]
 
 _lib = None
@@ -101,6 +101,8 @@ def load_library(path: str = LIB_PATH):
     lib.pd_debug_host_window_sums.argtypes = [C.c_void_p, C.c_uint32, C.c_uint64, C.c_uint64, C.POINTER(C.c_int64)]
     lib.pd_debug_device_window_sums.argtypes = lib.pd_debug_host_window_sums.argtypes
     lib.pd_debug_unify.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.POINTER(C.c_uint32), C.c_uint32, C.POINTER(PdResult)]
+    lib.pd_debug_candidates.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(C.c_int32), C.POINTER(C.c_uint8), C.POINTER(C.c_uint32),
+                                        C.POINTER(C.c_int32), C.c_uint64]
     lib.pd_contig_reserve_windows.argtypes = [C.c_void_p, C.c_uint64]
     lib.pd_shard_unique_id.argtypes = [C.POINTER(C.c_uint8)]
     lib.pd_shard_attach_nccl.argtypes = [C.c_void_p, C.POINTER(PdShardInfo), C.POINTER(C.c_uint8)]
@@ -398,6 +400,22 @@ class Scanner:
         if out["significant_windows"] is None:
             out["significant_windows"] = np.zeros(0, dtype=np.uint32)
         return out
+
+    def debug_candidates(self, q3: np.ndarray, state: np.ndarray):
+        """pd_debug_candidates: the candidate lengths (initialize_deletion_lengths) the scan's candidate step derives from
+        caller-built Q3 / state rows [n_windows, n_samples] (state 2 = the sample has a Q3) with this scanner's
+        thresholds. Returns one int32 array per window, ascending."""
+        q3 = np.ascontiguousarray(q3, dtype=np.int32)
+        state = np.ascontiguousarray(state, dtype=np.uint8)
+        assert q3.ndim == 2 and q3.shape == state.shape and q3.shape[1] == self.n_samples
+        nw = q3.shape[0]
+        counts = np.zeros(nw, dtype=np.uint32)
+        cap = max(int(np.count_nonzero(state == 2)), 1)          # a window has at most one length per sample with a Q3
+        cands = np.zeros(cap, dtype=np.int32)
+        self._check(self.lib.pd_debug_candidates(self.ctx, nw, q3.ctypes.data_as(C.POINTER(C.c_int32)),
+                                                 state.ctypes.data_as(C.POINTER(C.c_uint8)), counts.ctypes.data_as(C.POINTER(C.c_uint32)),
+                                                 cands.ctypes.data_as(C.POINTER(C.c_int32)), cap))
+        return np.split(cands[:int(counts.sum())], np.cumsum(counts.astype(np.int64))[:-1])
 
 
 def synth_read_group(seed: int, rg_index: int, mu: float, sigma: float, read_length: int, pairs_per_bp: float,

@@ -19,6 +19,16 @@
 constexpr uint32_t PD_FULL = 0xFFFFFFFFu;
 constexpr uint32_t PD_GRAN = 1024;                  // words per warp in k_stream; granule of the word -> tile index
 constexpr int PD_CAND_INLINE = 6;                   // candidate lengths kept inline per window job
+constexpr uint32_t PD_GRID_Y_MAX = 65535;           // CUDA's limit on gridDim.y and gridDim.z
+constexpr uint32_t PD_CAND_SMEM = 202 * 1024;       // bytes of Q3s k_candidates keeps in shared memory (one int per sample)
+
+// Launches over `rows` samples or read groups: gridDim.y is capped, gridDim.z takes the rest; the block's row is
+// pd_grid_row() (rows up to 65 535^2; blocks past the last row exit)
+inline dim3 pd_rows_grid(uint32_t x, uint32_t rows)
+{
+    const uint32_t y = rows < PD_GRID_Y_MAX ? (rows ? rows : 1u) : PD_GRID_Y_MAX;
+    return dim3(x, y, (rows + y - 1) / y);
+}
 
 // device counters of one scan (uint32 each)
 enum { CNT_TJOBS = 0, CNT_JOBS = 1, CNT_PAIRS = 2, CNT_POOL = 3, CNT_CALLS = 4, CNT_CJOBS = 5, CNT_ERR = 6, CNT_ALIVE = 7, CNT_KNOWN = 8, CNT_KJOBS = 9, CNT_N = 16 };
@@ -92,9 +102,11 @@ struct CandArgs {
     uint32_t * cjob_of;                 // [njobs] number of earlier windows of the batch with candidates (= candidate job)
     PdPair * pairs; uint32_t pair_cap;
     uint32_t * counters; unsigned long long * block_sums;
-    uint32_t npad;
+    uint32_t npad;                      // samples of the cohort, rounded up to a multiple of 32
     uint32_t force_sort;                // tests: always take the sorting path of k_candidates
     const uint8_t * job_dead;           // second screen stage: windows without any possible candidate (nullptr: stage off)
+    int32_t * sort_buf;                 // nullptr: k_candidates keeps the Q3s in shared memory; else [njobs][npad] for the
+                                        // sorting fallback of the instance that reads them from global memory
 };
 void pd_launch_q3(const PdDev & a, const GatherArgs & g, cudaStream_t st, uint64_t * launches);
 void pd_launch_screen2(const PdDev & a, const GatherArgs & g, cudaStream_t st, uint64_t * launches);
@@ -162,6 +174,8 @@ void pd_launch_emit(const EmitArgs & m, cudaStream_t st, uint64_t * launches);
 // ---------------------------------------------------------------------------------------------------------------
 // device helpers
 // ---------------------------------------------------------------------------------------------------------------
+__device__ __forceinline__ uint32_t pd_grid_row() { return blockIdx.z * gridDim.y + blockIdx.y; }      // see pd_rows_grid
+
 __device__ __forceinline__ PdTile load_tile(const PdTile * p)
 {
     const uint4 q = __ldg(reinterpret_cast<const uint4 *>(p));

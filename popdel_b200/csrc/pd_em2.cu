@@ -141,7 +141,8 @@ __global__ void __launch_bounds__(E2_T) k_e2_prep(PdDev a, EmArgs e, E2Args x)
     __shared__ uint32_t s_base;
     __shared__ unsigned long long s_ws[33];
     __shared__ uint32_t s_tile[E2_T / 32][32 * 33];
-    const uint32_t tid = threadIdx.x, sub = blockIdx.x, g = blockIdx.y;
+    const uint32_t tid = threadIdx.x, sub = blockIdx.x, g = pd_grid_row();
+    if (g >= a.R) return;
     const uint32_t p_lo = sub * E2_SUB, np = min((uint32_t)E2_SUB, e.npairs - p_lo);
     const uint32_t grp = g * x.nsub + sub;
     const size_t sbase = (size_t)grp * E2_SUB;
@@ -299,7 +300,8 @@ template <bool PASS_A>
 __global__ void __launch_bounds__(E2_T, E2_MINB) k_e2_reads(PdDev a, EmArgs e, E2Args x, uint32_t pass_no)
 {
     extern __shared__ double2 s_tab[];
-    const uint32_t tid = threadIdx.x, sub = blockIdx.x, g = blockIdx.y;
+    const uint32_t tid = threadIdx.x, sub = blockIdx.x, g = pd_grid_row();
+    if (g >= a.R) return;
     const uint32_t grp = g * x.nsub + sub;
     const uint32_t * nmaxs = x.blk_nmax + (size_t)grp * E2_WBS;
     const uint32_t * flags = x.wbflag + (size_t)grp * E2_WBS;
@@ -783,7 +785,8 @@ __global__ void __launch_bounds__(TPB) k_e2_pair(PdDev a, EmArgs e, E2Args x, ui
 __global__ void __launch_bounds__(E2_T, 4) k_e2_final_reads(PdDev a, EmArgs e, E2Args x)
 {
     extern __shared__ double2 s_tab[];                   // [rows] {log10, log10p}, then [rows] val (double)
-    const uint32_t tid = threadIdx.x, sub = blockIdx.x, g = blockIdx.y;
+    const uint32_t tid = threadIdx.x, sub = blockIdx.x, g = pd_grid_row();
+    if (g >= a.R) return;
     const uint32_t grp = g * x.nsub + sub;
     const uint32_t * nmaxs = x.blk_nmax + (size_t)grp * E2_WBS;
     const uint32_t * flags = x.finflag + (size_t)grp * E2_WBS;
@@ -1121,7 +1124,7 @@ int pd_launch_em2(pd_ctx * c, const PdDev & a, const EmArgs & e, double reads_pe
         PD_CUDA(c, cudaFuncSetAttribute(k_e2_reads<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_em));
     }
     if (smem_fin > 48 * 1024) PD_CUDA(c, cudaFuncSetAttribute(k_e2_final_reads, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_fin));
-    const dim3 gg(x.nsub, R);
+    const dim3 gg = pd_rows_grid(x.nsub, R);
     // pair phase: one warp per pair for cohorts of up to 128 samples, else one block per pair
     const uint32_t TP = N <= 128 ? 256 : (N <= 256 ? 256 : (N <= 512 ? 512 : 1024));
     const uint32_t gpb = N <= 128 ? 8 : 1;

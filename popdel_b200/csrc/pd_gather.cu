@@ -249,7 +249,7 @@ __global__ void __launch_bounds__(TQ_WARPS * 32, MINB) k_tile_q3(PdDev a, Gather
         }
         return;
     }
-    const uint32_t smp = blockIdx.y * TQ_WARPS + wib;
+    const uint32_t smp = pd_grid_row() * TQ_WARPS + wib;
     if (smp >= a.N) return;
     // (blocks walk several tile jobs: with the second screen stage most (tile job, sample) pairs have nothing to do)
     for (uint32_t tjb = blockIdx.x; tjb < ga.ntj; tjb += gridDim.x) q3_tile_job<TQ_ACT>(a, ga, sh_all[wib], lane, smp, tjb);
@@ -387,7 +387,7 @@ __global__ void __launch_bounds__(TG_WARPS * 32) k_tile_gather(PdDev a, GatherAr
 {
     __shared__ WarpStage stage_all[TG_WARPS];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-    const uint32_t smp = blockIdx.y * TG_WARPS + wib;
+    const uint32_t smp = pd_grid_row() * TG_WARPS + wib;
     if (smp >= a.N) return;
     const uint32_t wmask = ga.tj_cmask[blockIdx.x];                       // windows of the tile with candidate lengths
     const uint32_t cfirst = ga.tj_cfirst[blockIdx.x];
@@ -499,35 +499,58 @@ __device__ __forceinline__ bool bits_any(const uint32_t * bits, uint32_t lo, uin
     return r != 0;
 }
 
+// f(Q3) of every sample of window `job` that has one (state 2), samples strided over the block's threads
+template <typename F>
+__device__ __forceinline__ void for_window_q3(const CandArgs & ca, uint32_t job, F f)
+{
+    for (uint32_t p = 0; p < ca.nparts; ++p) {
+        const uint32_t np = ca.part_n[p];
+        const uint8_t * ss = ca.sstat[p] + (size_t)job * np;
+        const int32_t * qq = ca.q3[p] + (size_t)job * np;
+        for (uint32_t s = threadIdx.x; s < np; s += blockDim.x)
+            if (ss[s] == 2) f(qq[s]);
+    }
+}
+
 // One block per flagged window: initialize_deletion_lengths (genotype_deletion_popdel_call.h:58-86) WITHOUT sorting the
 // Q3 values. The chain clusters (sorted neighbours closer than 50) are the maximal runs of a presence bitmap over the
 // value range whose gaps are shorter than 50: a value is the top of a cluster iff none of the next 49 values is
 // present. Per cluster: sum and count by shared-memory atomics; the ranks of its members in the sorted array are
 // [number of smaller values, + count), which is all the rank-indexed thresholds need (quirk, :65,72,80). Falls back to
 // the bitonic sort for value ranges beyond 65 536 or more than 1 024 clusters.
+// GLOBAL = false: the window's Q3s are copied once into dynamic shared memory (one int per sample of the cohort).
+// GLOBAL = true (cohorts whose Q3s do not fit shared memory): every pass re-reads them from the Q3 / state rows in global
+// memory; only the sorting fallback copies them, into this window's row of ca.sort_buf.
+template <bool GLOBAL>
 __global__ void __launch_bounds__(256) k_candidates(PdDev a, CandArgs ca, int mode)
 {
-    extern __shared__ int32_t sv[];
+    extern __shared__ int32_t s_q3[];
     __shared__ uint32_t s_bits[CAND_BITS / 32 + 4];
     __shared__ int32_t s_top[CAND_TOPS], s_sorted[CAND_TOPS], s_sum[CAND_TOPS];
     __shared__ uint32_t s_cnt[CAND_TOPS];
-    __shared__ uint32_t s_n, s_ntop, s_thr;
+    __shared__ uint32_t s_n, s_ntop, s_thr, s_fill;
     __shared__ int32_t s_min, s_max;
     const uint32_t job = blockIdx.x;
+    int32_t * const sv = GLOBAL ? ca.sort_buf + (size_t)job * ca.npad : s_q3;
     if (mode == 1 && ca.cand_cnt[job] <= (uint32_t)PD_CAND_INLINE) return;
     if (ca.job_dead && ca.job_dead[job]) { if (threadIdx.x == 0 && mode == 0) ca.cand_cnt[job] = 0; return; }      // rejected by the second screen stage
-    if (threadIdx.x == 0) { s_n = 0; s_ntop = 0; s_min = INT_MAX; s_max = INT_MIN; }
+    if (threadIdx.x == 0) { s_n = 0; s_ntop = 0; s_min = INT_MAX; s_max = INT_MIN; if (GLOBAL) s_fill = 0; }
     __syncthreads();
-    for (uint32_t p = 0; p < ca.nparts; ++p) {
-        const uint32_t np = ca.part_n[p];
-        const uint8_t * ss = ca.sstat[p] + (size_t)job * np;
-        const int32_t * qq = ca.q3[p] + (size_t)job * np;
-        for (uint32_t s = threadIdx.x; s < np; s += blockDim.x)
-            if (ss[s] == 2) { const int32_t v = qq[s]; sv[atomicAdd(&s_n, 1u)] = v; atomicMin(&s_min, v); atomicMax(&s_max, v); }
+    if (GLOBAL) {
+        uint32_t n = 0; int32_t lo = INT_MAX, hi = INT_MIN;
+        for_window_q3(ca, job, [&](int32_t v) { ++n; lo = min(lo, v); hi = max(hi, v); });
+        if (n) { atomicAdd(&s_n, n); atomicMin(&s_min, lo); atomicMax(&s_max, hi); }
+    } else {
+        for_window_q3(ca, job, [&](int32_t v) { sv[atomicAdd(&s_n, 1u)] = v; atomicMin(&s_min, v); atomicMax(&s_max, v); });
     }
     __syncthreads();
     const uint32_t nv = s_n;
     if (nv == 0) { if (threadIdx.x == 0 && mode == 0) ca.cand_cnt[job] = 0; return; }
+    // f(v) for every Q3 of the window, values strided over the block's threads
+    auto each_value = [&](auto f) {
+        if (GLOBAL) for_window_q3(ca, job, f);
+        else for (uint32_t i = threadIdx.x; i < nv; i += blockDim.x) f(sv[i]);
+    };
     CandEmit emit{ca, job, mode, mode == 1 ? ca.cand_off[job] : 0u, 0u};
     const int32_t mn = s_min;
     const uint32_t range = (uint32_t)(s_max - mn) + 1u;
@@ -536,7 +559,7 @@ __global__ void __launch_bounds__(256) k_candidates(PdDev a, CandArgs ca, int mo
         const uint32_t nwords = (range + 31) / 32;
         for (uint32_t w = threadIdx.x; w < nwords + 3; w += blockDim.x) s_bits[w] = 0;
         __syncthreads();
-        for (uint32_t i = threadIdx.x; i < nv; i += blockDim.x) { const uint32_t b = (uint32_t)(sv[i] - mn); atomicOr(&s_bits[b >> 5], 1u << (b & 31u)); }
+        each_value([&](int32_t v) { const uint32_t b = (uint32_t)(v - mn); atomicOr(&s_bits[b >> 5], 1u << (b & 31u)); });
         __syncthreads();
         for (uint32_t w = threadIdx.x; w < nwords; w += blockDim.x)
             for (uint32_t m = s_bits[w]; m; m &= m - 1) {
@@ -555,12 +578,12 @@ __global__ void __launch_bounds__(256) k_candidates(PdDev a, CandArgs ca, int mo
             s_sorted[r] = v; s_sum[t] = 0; s_cnt[t] = 0;
         }
         __syncthreads();
-        for (uint32_t i = threadIdx.x; i < nv; i += blockDim.x) {
-            const int32_t b = sv[i] - mn;
+        each_value([&](int32_t v) {
+            const int32_t b = v - mn;
             uint32_t lo = 0, hi = K - 1;                               // smallest k with top_k >= b
             while (lo < hi) { const uint32_t mid = (lo + hi) >> 1; if (s_sorted[mid] >= b) hi = mid; else lo = mid + 1; }
-            atomicAdd(&s_sum[lo], sv[i]); atomicAdd(&s_cnt[lo], 1u);
-        }
+            atomicAdd(&s_sum[lo], v); atomicAdd(&s_cnt[lo], 1u);
+        });
         __syncthreads();
         uint32_t r0 = 0;
         for (uint32_t k = 0; k < K; ++k) {
@@ -583,7 +606,11 @@ __global__ void __launch_bounds__(256) k_candidates(PdDev a, CandArgs ca, int mo
     }
     // ---- fallback: bitonic sort, then the reference's linear pass. Every compare-exchange sorts ascending (the first step
     // of a merge pairs i with its mirror image inside the block), so the padding up to the next power of two is virtual:
-    // a partner at or beyond nv stands for +infinity and never moves -- shared memory holds nv values, not a power of two.
+    // a partner at or beyond nv stands for +infinity and never moves -- sv holds nv values, not a power of two.
+    if (GLOBAL) {                                                     // (in any order: the sort decides it)
+        for_window_q3(ca, job, [&](int32_t v) { sv[atomicAdd(&s_fill, 1u)] = v; });
+        __syncthreads();
+    }
     uint32_t np2 = 1; while (np2 < nv) np2 <<= 1;
     for (uint32_t k = 2; k <= np2; k <<= 1)
         for (uint32_t j = k >> 1; j > 0; j >>= 1) {
@@ -667,7 +694,7 @@ void pd_launch_q3(const PdDev & a, const GatherArgs & g, cudaStream_t st, uint64
         ++*launches;
         return;
     }
-    k_tile_q3<48, 9><<<dim3(gx, (a.N + TQ_WARPS - 1) / TQ_WARPS), TQ_WARPS * 32, 0, st>>>(a, g);
+    k_tile_q3<48, 9><<<pd_rows_grid(gx, (a.N + TQ_WARPS - 1) / TQ_WARPS), TQ_WARPS * 32, 0, st>>>(a, g);
     ++*launches;
 }
 
@@ -685,21 +712,24 @@ void pd_launch_cmask(const GatherArgs & g, const CandArgs & ca, uint32_t * tj_cm
 
 void pd_launch_gather(const PdDev & a, const GatherArgs & g, cudaStream_t st, uint64_t * launches)
 {
-    k_tile_gather<<<dim3(g.ntj, (a.N + TG_WARPS - 1) / TG_WARPS), TG_WARPS * 32, 0, st>>>(a, g);
+    k_tile_gather<<<pd_rows_grid(g.ntj, (a.N + TG_WARPS - 1) / TG_WARPS), TG_WARPS * 32, 0, st>>>(a, g);
     ++*launches;
 }
 
 int pd_launch_candidates(pd_ctx * c, const PdDev & a, const CandArgs & ca, cudaStream_t st, uint64_t * launches)
 {
-    if ((size_t)ca.npad * 4 > 48 * 1024)
-        PD_CUDA(c, cudaFuncSetAttribute(k_candidates, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(ca.npad * 4)));
+    const bool global = ca.sort_buf != nullptr;
+    if (!global && (size_t)ca.npad * 4 > 48 * 1024)
+        PD_CUDA(c, cudaFuncSetAttribute(k_candidates<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(ca.npad * 4)));
     const uint32_t threads = ca.npad >= 512 ? 256 : (ca.npad >= 128 ? 64 : 32);
     const uint32_t nb = (ca.njobs + 1023) / 1024;
-    k_candidates<<<ca.njobs, threads, ca.npad * 4, st>>>(a, ca, 0);
+    if (global) k_candidates<true><<<ca.njobs, threads, 0, st>>>(a, ca, 0);
+    else k_candidates<false><<<ca.njobs, threads, ca.npad * 4, st>>>(a, ca, 0);
     k_cand_sums<<<nb, 1024, 0, st>>>(ca);
     k_cand_offsets<<<1, 1024, 0, st>>>(ca, nb);
     k_cand_write<<<nb, 1024, 0, st>>>(ca);
-    k_candidates<<<ca.njobs, threads, ca.npad * 4, st>>>(a, ca, 1);
+    if (global) k_candidates<true><<<ca.njobs, threads, 0, st>>>(a, ca, 1);
+    else k_candidates<false><<<ca.njobs, threads, ca.npad * 4, st>>>(a, ca, 1);
     *launches += 5;
     PD_CUDA(c, cudaGetLastError());
     return 0;

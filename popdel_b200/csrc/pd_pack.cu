@@ -650,9 +650,13 @@ int pd_pack_on_device(pd_ctx * c)
         PD_CUDA(c, cudaStreamWaitEvent(st, c->ev_pack[k], 0));
         a.g0 = grp_lo[k]; a.ng = grp_lo[k + 1] - grp_lo[k];
         const uint64_t nt_grp = per * a.ng;
-        if (any_compact && grp_max[k])           // (read groups pushed as raw arrays have no blocks: their chunks exit at once)
-            k_expand_compact<<<dim3((unsigned)((grp_max[k] + 4095) / 4096), a.ng), 256, 0, st>>>(d_lo, d_d24, d_blk, d_rg_start, d_blk_start, d_nblk, a.g0, d_pos, d_dev);
-        if (grp_max[k]) k_check_span<<<dim3((unsigned)((grp_max[k] + 1023) / 1024), a.ng), 256, 0, st>>>(a);
+        for (uint32_t g = 0; g < a.ng; g += 65535) {                     // (gridDim.y: at most 65 535 read groups per launch)
+            PackArgs b = a;
+            b.g0 = a.g0 + g; b.ng = std::min<uint32_t>(a.ng - g, 65535);
+            if (any_compact && grp_max[k])       // (read groups pushed as raw arrays have no blocks: their chunks exit at once)
+                k_expand_compact<<<dim3((unsigned)((grp_max[k] + 4095) / 4096), b.ng), 256, 0, st>>>(d_lo, d_d24, d_blk, d_rg_start, d_blk_start, d_nblk, b.g0, d_pos, d_dev);
+            if (grp_max[k]) k_check_span<<<dim3((unsigned)((grp_max[k] + 1023) / 1024), b.ng), 256, 0, st>>>(b);
+        }
         k_tile_first<<<(unsigned)((nt_grp + 255) / 256), 256, 0, st>>>(a);
         k_cap_check<<<a.ng * chunks, 1024, 0, st>>>(a, chunks);
         k_tile_offsets<<<a.ng, 1024, 0, st>>>(a, d_rel, d_rg_words);

@@ -19,7 +19,7 @@ namespace {
 enum Slot {                                     // d_scratch slots
     S_NEED = 0, S_TFLAGS, S_COUNTERS, S_TJ_TILE, S_TJ_MASK, S_TJ_WBASE, S_JOBWIN, S_BSUMS,
     S_ACT_OFF, S_ACT_CNT, S_Q3, S_SSTAT, S_CAND_CNT, S_CAND_INL, S_CAND_OFF, S_CJOB_OF, S_TJ_CMASK, S_TJ_CFIRST, S_PAIRS, S_POOL_POS, S_POOL_DEV,
-    S_DLX, S_DLE, S_SHIFTS, S_STATES, S_PS0, S_PS1, S_CALLS0, S_CALLS1, S_VALID0, S_VALID1, S_DONE0, S_DONE1, S_CHUNK_BASE, S_DBG, S_DMAX, S_ALL_Q3, S_ALL_SS,
+    S_DLX, S_DLE, S_SHIFTS, S_STATES, S_PS0, S_PS1, S_CALLS0, S_CALLS1, S_VALID0, S_VALID1, S_DONE0, S_DONE1, S_CHUNK_BASE, S_DBG, S_DMAX, S_ALL_Q3, S_ALL_SS, S_CAND_SORT,
     S_KNOWN = 64, S_TJ_ALIVE, S_JOB_DEAD, S_KJOBS, S_TJ_OF_TILE
 };
 
@@ -127,6 +127,17 @@ int ensure_results(pd_ctx * c, size_t need_calls, size_t row, size_t keep_calls)
         c->res_ps = p; c->cap_res_ps = want;
     }
     return 0;
+}
+
+// Samples of the cohort rounded up to a multiple of 32 (k_candidates' shared-memory row of Q3s and its block size)
+uint32_t cand_npad(uint32_t n_global) { return (std::max<uint32_t>(n_global, 32) + 31u) & ~31u; }
+
+// The instance of k_candidates that reads the Q3s from global memory: for cohorts whose Q3s do not fit its shared memory,
+// or at any size with PD_CAND_GLOBAL=1 (tests: both instances on the same input)
+bool cand_global(uint32_t npad)
+{
+    const char * e = getenv("PD_CAND_GLOBAL");
+    return (size_t)npad * 4 > PD_CAND_SMEM || (e && atoi(e) != 0);
 }
 
 }  // namespace
@@ -238,7 +249,9 @@ int pd_run_scan(pd_ctx * c, uint64_t first_window, uint64_t n_windows, pd_result
 
     // ---- genotyping stage. Level 1: batches of tile jobs (Q3 of every flagged window, candidates). Level 2: the windows
     // with candidates ("candidate jobs") in sub-batches of whole tiles (active-set pool, EM, final pass, emission).
-    const size_t job_bytes = 9ull * Nb * (sh ? sh->world + 1 : 1) + 4ull * (PD_CAND_INLINE + 3) + 8;
+    const uint32_t npad = cand_npad(Ng);
+    const bool cglobal = cand_global(npad);
+    const size_t job_bytes = 9ull * Nb * (sh ? sh->world + 1 : 1) + (cglobal ? 4ull * npad : 0) + 4ull * (PD_CAND_INLINE + 3) + 8;
     uint32_t JB = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(3000000000ull / job_bytes, 64), 1u << 20);
     if (getenv("PD_JOB_BATCH")) JB = std::max<uint32_t>((uint32_t)atoi(getenv("PD_JOB_BATCH")), 64);           // test knobs
     const uint32_t rows_env = getenv("PD_CJOB_ROWS") ? std::max<uint32_t>((uint32_t)atoi(getenv("PD_CJOB_ROWS")), 1) : 0;
@@ -251,8 +264,6 @@ int pd_run_scan(pd_ctx * c, uint64_t first_window, uint64_t n_windows, pd_result
         PD_CUDA(c, cudaMemcpyAsync(h_wbase.data(), j.tj_wbase, (size_t)n_tj * 4, cudaMemcpyDeviceToHost, st));
         PD_CUDA(c, cudaStreamSynchronize(st));
     }
-    const uint32_t npad = (std::max<uint32_t>(Ng, 32) + 31u) & ~31u;   // Q3 of every sample of the cohort in shared memory (k_candidates)
-    if ((size_t)npad * 4 > 202 * 1024) return pd_fail(c, PD_ERR_CAPACITY, "more than 51 700 samples per cohort: the candidate step keeps one Q3 per sample in shared memory");
     const bool em2 = !sh && pd_em2_usable(c);                          // sample-major pipeline (pd_em2.cu)
     // (reads per pair are not known before the gather: budget 40 active read pairs per read group)
     const size_t pair_bytes = 48ull * Nb + 4ull * Rb + 2 * 52ull * Nb + 128 + (em2 ? pd_em2_pair_bytes(Rb, 40.0 * Rb) : 0);
@@ -319,6 +330,7 @@ int pd_run_scan(pd_ctx * c, uint64_t first_window, uint64_t n_windows, pd_result
         ca.nparts = 1; ca.q3[0] = ga.q3; ca.sstat[0] = ga.sstat; ca.part_n[0] = N; ca.min_init = c->d_min_init;
         ca.njobs = nj; ca.job_base = job_base; ca.counters = d_counters; ca.block_sums = d_bsums; ca.npad = npad;
         ca.force_sort = (slow_env >> 2) & 1u;
+        if (cglobal && grow_scratch(c, S_CAND_SORT, ca.sort_buf, (size_t)nj * npad)) return c->status;
         ca.job_dead = screen2 ? ga.job_dead : nullptr;
         int32_t * all_q3 = nullptr; uint8_t * all_ss = nullptr;
         if (sh) {
@@ -604,5 +616,62 @@ extern "C" int pd_debug_unify(pd_ctx * c, uint64_t n, const pd_call * calls, con
     out->calls = c->res_calls;
     out->per_sample = c->res_ps;
     out->significant_windows = c->res_sig;
+    return 0;
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// device-side validation hook: the candidate step (pd_launch_candidates) on caller-built Q3 / state rows
+// ---------------------------------------------------------------------------------------------------------
+extern "C" int pd_debug_candidates(pd_ctx * c, uint64_t n_windows, const int32_t * q3, const uint8_t * state, uint32_t * counts,
+                                   int32_t * cands, uint64_t cap)
+{
+    if (!c || (n_windows && (!q3 || !state || !counts)) || (cap && !cands)) return PD_ERR_ARG;
+    if (c->status) return c->status;
+    if (c->device < 0) return pd_fail(c, PD_ERR_ARG, "pd_debug_candidates: host-only context (device = -1)");
+    if (c->shard) return pd_fail(c, PD_ERR_ARG, "pd_debug_candidates: sample-sharded context (the probe takes one context's Q3 rows)");
+    if (n_windows > 0x7FFFFFFFull) return pd_fail(c, PD_ERR_ARG, "pd_debug_candidates: more than 2^31 - 1 windows");
+    if (n_windows == 0) return 0;
+    PD_CUDA(c, cudaSetDevice(c->device));
+    cudaStream_t st = c->stream;
+    const uint32_t nj = (uint32_t)n_windows, N = c->N, npad = cand_npad(N);
+    PdDev a{};
+    a.N = N; a.R = c->R; a.t_min = c->t_min;
+    CandArgs ca;
+    memset(&ca, 0, sizeof(ca));
+    int32_t * d_q3; uint8_t * d_ss;
+    if (grow_scratch(c, S_Q3, d_q3, (size_t)nj * N)) return c->status;
+    if (grow_scratch(c, S_SSTAT, d_ss, (size_t)nj * N)) return c->status;
+    PD_CUDA(c, cudaMemcpyAsync(d_q3, q3, (size_t)nj * N * 4, cudaMemcpyHostToDevice, st));
+    PD_CUDA(c, cudaMemcpyAsync(d_ss, state, (size_t)nj * N, cudaMemcpyHostToDevice, st));
+    ca.nparts = 1; ca.q3[0] = d_q3; ca.sstat[0] = d_ss; ca.part_n[0] = N; ca.min_init = c->d_min_init;
+    ca.njobs = nj; ca.job_base = 0; ca.npad = npad;
+    ca.force_sort = ((getenv("PD_FORCE_SLOW") ? (uint32_t)atoi(getenv("PD_FORCE_SLOW")) : 0u) >> 2) & 1u;
+    if (cand_global(npad) && grow_scratch(c, S_CAND_SORT, ca.sort_buf, (size_t)nj * npad)) return c->status;
+    if (grow_scratch(c, S_COUNTERS, ca.counters, (size_t)CNT_N)) return c->status;
+    if (grow_scratch(c, S_BSUMS, ca.block_sums, (size_t)(nj + 1023) / 1024 + 1)) return c->status;
+    if (grow_scratch(c, S_CAND_CNT, ca.cand_cnt, (size_t)nj)) return c->status;
+    if (grow_scratch(c, S_CAND_INL, ca.cand_inline, (size_t)nj * PD_CAND_INLINE)) return c->status;
+    if (grow_scratch(c, S_CAND_OFF, ca.cand_off, (size_t)nj)) return c->status;
+    if (grow_scratch(c, S_CJOB_OF, ca.cjob_of, (size_t)nj)) return c->status;
+    size_t pair_cap = std::max<size_t>(c->cap_scratch[S_PAIRS] / sizeof(PdPair), (size_t)nj * 2 + 1024);
+    uint32_t cnt[CNT_N];
+    uint64_t launches = 0;
+    for (int attempt = 0; ; ++attempt) {                              // (a second attempt has the exact size)
+        if (grow_scratch(c, S_PAIRS, ca.pairs, pair_cap)) return c->status;
+        ca.pair_cap = (uint32_t)std::min<size_t>(pair_cap, 0xFFFFFFF0ull);
+        if (pd_launch_candidates(c, a, ca, st, &launches)) return c->status;
+        PD_CUDA(c, cudaMemcpyAsync(cnt, ca.counters, sizeof(cnt), cudaMemcpyDeviceToHost, st));
+        PD_CUDA(c, cudaStreamSynchronize(st));
+        if (cnt[CNT_PAIRS] <= ca.pair_cap) break;
+        if (attempt == 1) return pd_fail(c, PD_ERR_CAPACITY, "pd_debug_candidates: candidate list overflow");
+        pair_cap = (size_t)cnt[CNT_PAIRS] + 1024;
+    }
+    const uint32_t total = cnt[CNT_PAIRS];
+    std::vector<PdPair> pairs(total);
+    PD_CUDA(c, cudaMemcpyAsync(counts, ca.cand_cnt, (size_t)nj * 4, cudaMemcpyDeviceToHost, st));
+    if (total) PD_CUDA(c, cudaMemcpyAsync(pairs.data(), ca.pairs, (size_t)total * sizeof(PdPair), cudaMemcpyDeviceToHost, st));
+    PD_CUDA(c, cudaStreamSynchronize(st));
+    for (uint64_t i = 0; i < std::min<uint64_t>(total, cap); ++i) cands[i] = pairs[i].L0;
+    if (total > cap) return pd_fail(c, PD_ERR_CAPACITY, "pd_debug_candidates: more candidate lengths than `cap`");
     return 0;
 }

@@ -155,7 +155,8 @@ __global__ void __launch_bounds__(256) k_count(PdDev a, ScreenArgs s)
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const uint32_t wq = blockIdx.x * 8 + wib;
     if (wq >= s.need_stride) return;
-    const uint32_t smp = blockIdx.y;
+    const uint32_t smp = pd_grid_row();                             // (samples over grid y and z: pd_rows_grid)
+    if (smp >= a.N) return;
     uint32_t mq = s.need[(size_t)smp * s.need_stride + wq];
     if (mq == 0) return;
     const uint32_t g0 = a.sample_rg[smp], g1 = a.sample_rg[smp + 1];
@@ -303,7 +304,7 @@ void pd_launch_screen(const PdDev & a, const ScreenArgs & s, uint32_t max_rg_wor
     ++*launches;
     cudaEventRecord(after_stream, st);
     if (s.total_longs) { k_mark_long<<<(s.total_longs + 255) / 256, 256, 0, st>>>(a, s); ++*launches; }
-    k_count<<<dim3((s.need_stride + 7) / 8, a.N), 256, 0, st>>>(a, s);
+    k_count<<<pd_rows_grid((s.need_stride + 7) / 8, a.N), 256, 0, st>>>(a, s);
     ++*launches;
 }
 
